@@ -40,6 +40,7 @@ def parse():
   p.add_argument('--no-e2e', action='store_true')
   p.add_argument('--no-cpu-baseline', action='store_true')
   p.add_argument('--ref-steps-per-step', type=int, default=10, help='reference arm: oracle loop iterations per bench step and worker')
+  p.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write what the last one computed (rank 0) to DIR/<name>.npy, float32, < 64 MB in all')
   return p.parse_args()
 
 
@@ -195,6 +196,7 @@ def run_b200(a):
   ms, launches = timed(K)
   clk = clocks.stop()
   value = R * world * K / (ms / 1e3)
+  if a.dump_outputs and rank == 0: dump_outputs(tr, a.dump_outputs)  # before the diagnostics below run further steps
 
   # ---- per-kernel roofline of the dominant kernel (the dense 256x256 grouped GEMMs), measured with CUDA events around
   # each launch on the launching stream during 2 extra eager steps
@@ -241,6 +243,29 @@ def run_b200(a):
                 gemm_mode=a.gemm_mode, eval=ev, strong=strong)
     print(json.dumps(line), flush=True)
   distributed.barrier()
+
+
+DUMP_LIMIT = 1 << 21  # entries kept per array; at most four arrays (the parameter buffers) exceed it, so a dump stays well under 64 MB
+
+
+def dump_outputs(tr, out_dir):
+  """Writes what the last train_step computed, as its caller reads it, to <out_dir>/<name>.npy (float32): the SAC and
+  discriminator results of the step, the relabelled rewards of its batch, the last episode returns, log_alpha and the
+  parameter buffers ([replicas, P]) the step left behind. An array above DUMP_LIMIT entries keeps a fixed, seeded sample
+  of its flattened entries, at the same positions for any build with the same shapes."""
+  import numpy as np
+  import torch
+  torch.cuda.synchronize()
+  arrays = dict(sac_log_probs=tr.sac_out['log_probs'], sac_q_values=tr.sac_out['q_values'], sac_losses=tr.sac_out['losses'], gail_losses=tr.gail_losses,
+                batch_rewards=tr.batch['rewards'], last_return=tr.last_return, log_alpha=tr.log_alpha)
+  for name, mod in (('actor', tr.actor), ('critic', tr.critic), ('target_critic', tr.target_critic), ('discriminator', tr.discriminator)):
+    params = mod.parameters() if hasattr(mod, 'parameters') else []
+    if params: arrays[f'{name}_params'] = torch.cat([p.reshape(-1) for p in params])
+  os.makedirs(out_dir, exist_ok=True)
+  for name, t in arrays.items():
+    v = t.detach().float().cpu().numpy()
+    if v.size > DUMP_LIMIT: v = v.reshape(-1)[np.sort(np.random.default_rng(v.size).choice(v.size, DUMP_LIMIT, replace=False))]
+    np.save(os.path.join(out_dir, f'{name}.npy'), v)
 
 
 def measure_eval(tr, a, world):

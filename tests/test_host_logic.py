@@ -1,5 +1,6 @@
 """CPU-only checks of the host-side logic of the drop-in: expert-data ingest (environments.py:63-125), the Hydra-free
 configuration surface (train.py:21-23, conf/) and the replica sharding helpers. No CUDA call is made here."""
+import json
 import os
 
 import numpy as np
@@ -8,7 +9,7 @@ import torch
 import yaml
 
 from il_b200 import config, environments
-from oracle import cases, port, refstub
+from oracle import cases, port
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 INGEST = [n for n, c in cases.CASES.items() if c['kind'] == 'ingest']
@@ -57,11 +58,6 @@ def test_expert_ingest_edge_cases():
   assert sub['states'].shape[0] == 2 and torch.equal(sub['weights'], torch.full((2,), 1 / 20))
 
 
-def _reference_conf(*parts):
-  path = os.path.join(refstub.REFERENCE_DIR, 'conf', *parts)
-  with open(path) as f: return yaml.safe_load(f)
-
-
 def _flat(d, prefix=''):
   out = {}
   for k, v in d.items():
@@ -89,47 +85,83 @@ def test_config_defaults_and_overrides():
   with pytest.raises(AttributeError): _ = cfg.training.no_such_key
 
 
-@pytest.mark.skipif(not refstub.available(), reason='reference tree not present (GPU box)')
+CONF_FILES = (['train_config.yaml'] + [f'algorithm/{alg}.yaml' for alg in ('SAC', 'GAIL', 'GMMIL', 'PWIL', 'BC')]
+              + [f'optimised_hyperparameters/{alg}_{n}_trajectories.yaml' for alg in ('BC', 'GAIL', 'GMMIL', 'PWIL') for n in (5, 10, 25)])
+INIT_SEED, INIT_REPLICAS, INIT_DIMS = 7, 3, (12, 3, 256)  # S, A, H
+INIT_SAMPLES, INIT_ATOL = 32, 1e-6  # orthogonal_ goes through a QR factorisation whose last bits follow the thread count and the CPU's LAPACK path
+
+
+def _golden_json(name):
+  with open(os.path.join(ROOT, 'tests', 'golden', name)) as f: return json.load(f)
+
+
+def _init_idx(size):
+  return np.random.RandomState(size).choice(size, min(size, INIT_SAMPLES), replace=False)
+
+
+def _init_record(t):
+  v = t.detach().double().reshape(-1)
+  return dict(shape=list(t.shape), sample=v[_init_idx(v.numel())].tolist(), sum=float(v.sum()), absmax=float(v.abs().max()))
+
+
+def record_reference_conf(conf_dir):
+  """The values of the reference's conf/ files listed in CONF_FILES, flattened, without Hydra's own keys
+  (tests/golden/reference_conf.json, written by `python -m oracle.make_golden reference_conf`)."""
+  out = {}
+  for name in CONF_FILES:
+    with open(os.path.join(conf_dir, *name.split('/'))) as f: d = yaml.safe_load(f) or {}
+    out[name] = _flat({k: v for k, v in d.items() if k not in ('defaults', 'hydra')})
+  return out
+
+
+def record_reference_init(ref):
+  """Shape, a fixed sample of entries, sum and max |x| of every initial parameter of the reference's SoftActor and TwinCritic built after
+  torch.manual_seed(INIT_SEED + r) (train.py:51-66), r < INIT_REPLICAS (tests/golden/reference_init.json, written by
+  `python -m oracle.make_golden reference_init`)."""
+  S, A, H = INIT_DIMS
+  mc = ref.DictConfig(hidden_size=H, depth=2, activation='relu')
+  out = {}
+  for r in range(INIT_REPLICAS):
+    torch.manual_seed(INIT_SEED + r)
+    actor, critic = ref.models.SoftActor(S, A, mc), ref.models.TwinCritic(S, A, mc)
+    for name, seq in (('actor', actor.actor), ('critic_1', critic.critic_1.critic), ('critic_2', critic.critic_2.critic)):
+      out[f'{r}/{name}'] = [_init_record(t) for lin in seq if isinstance(lin, torch.nn.Linear) for t in (lin.weight, lin.bias)]
+  return out
+
+
 def test_conf_tree_carries_the_reference_values():
   """Every key of the reference's train_config.yaml / algorithm overlays / tuned overlays that this repo ships has
   the reference's value (this repo adds keys — replicas, device_rng, cuda_graphs, gemm_mode, output_dir — never changes one)."""
+  ref = _golden_json('reference_conf.json')
+  assert sorted(ref) == sorted(CONF_FILES)
   ours = _flat(config.load_config([]))
-  for k, v in _flat(_reference_conf('train_config.yaml')).items():
-    if k.startswith(('hydra', 'defaults')): continue
+  for k, v in ref['train_config.yaml'].items():
     assert k in ours, f'train_config.yaml: {k} missing'
     assert ours[k] == v, (k, ours[k], v)
-  for alg in ('SAC', 'GAIL', 'GMMIL', 'PWIL', 'BC'):
-    with open(os.path.join(ROOT, 'conf', 'algorithm', f'{alg}.yaml')) as f: mine = _flat(yaml.safe_load(f) or {})
-    theirs = _flat({k: v for k, v in (_reference_conf('algorithm', f'{alg}.yaml') or {}).items() if k not in ('defaults', 'hydra')})
-    assert mine == theirs, (alg, set(mine.items()) ^ set(theirs.items()))
-  for alg in ('BC', 'GAIL', 'GMMIL', 'PWIL'):
-    for n in (5, 10, 25):
-      name = f'{alg}_{n}_trajectories.yaml'
-      with open(os.path.join(ROOT, 'conf', 'optimised_hyperparameters', name)) as f: mine = _flat(yaml.safe_load(f) or {})
-      theirs = _flat({k: v for k, v in (_reference_conf('optimised_hyperparameters', name) or {}).items() if k not in ('defaults', 'hydra')})
-      assert mine == theirs, (name, set(mine.items()) ^ set(theirs.items()))
+  for name in CONF_FILES[1:]:
+    with open(os.path.join(ROOT, 'conf', *name.split('/'))) as f: mine = _flat(yaml.safe_load(f) or {})
+    assert mine == ref[name], (name, mine, ref[name])
 
 
-@pytest.mark.skipif(not refstub.available(), reason='reference tree not present (GPU box)')
 def test_parameter_initialisation_consumes_the_reference_rng_stream():
   """train.py:51-66 seeds torch once and builds actor, then the twin critic; replica r of this build must initialise
   like a reference run with seed + r (net.ReplicaRNG + net.init_fcnn_params, CPU side of ReplicaMLP)."""
   from il_b200 import net
-  ref = refstub.load()
-  S, A, H = 12, 3, 256
-  mc = ref.DictConfig(hidden_size=H, depth=2, activation='relu')
-  rng = net.ReplicaRNG(seed=7, replicas=3)
-  for r in range(3):
-    torch.manual_seed(7 + r)
-    actor, critic = ref.models.SoftActor(S, A, mc), ref.models.TwinCritic(S, A, mc)
+  want = _golden_json('reference_init.json')
+  S, A, H = INIT_DIMS
+  rng = net.ReplicaRNG(seed=INIT_SEED, replicas=INIT_REPLICAS)
+  for r in range(INIT_REPLICAS):
     with rng.replica(r):
       mine_actor = net.init_fcnn_params([S, H, H, 2 * A], 'relu')
       mine_c1, mine_c2 = net.init_fcnn_params([S + A, H, H, 1], 'relu'), net.init_fcnn_params([S + A, H, H, 1], 'relu')
-    for mine, theirs in ((mine_actor, actor.actor), (mine_c1, critic.critic_1.critic), (mine_c2, critic.critic_2.critic)):
-      lins = [m for m in theirs if isinstance(m, torch.nn.Linear)]
-      assert len(lins) * 2 == len(mine)
-      for l, lin in enumerate(lins):
-        assert torch.equal(mine[2 * l], lin.weight.detach()) and torch.equal(mine[2 * l + 1], lin.bias.detach())
+    for name, mine in (('actor', mine_actor), ('critic_1', mine_c1), ('critic_2', mine_c2)):
+      theirs = want[f'{r}/{name}']
+      assert len(theirs) == len(mine) == 6, (r, name)
+      for i, (t, ref) in enumerate(zip(mine, theirs)):
+        got, where = _init_record(t), f'replica {r} {name} parameter {i}'
+        assert got['shape'] == ref['shape'], where
+        assert np.abs(np.subtract(got['sample'], ref['sample'])).max() <= INIT_ATOL, where
+        assert abs(got['sum'] - ref['sum']) <= INIT_ATOL * t.numel() and abs(got['absmax'] - ref['absmax']) <= INIT_ATOL, where
   # the global stream is left untouched by the per-replica streams
   torch.manual_seed(123)
   a = torch.rand(3)
