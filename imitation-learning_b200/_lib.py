@@ -28,7 +28,8 @@ class Mlp(C.Structure):
 
 
 class Adam(C.Structure):
-  _fields_ = [('m', vp), ('v', vp), ('step', vp), ('lr', C.c_double), ('beta1', C.c_double), ('beta2', C.c_double), ('eps', C.c_double), ('weight_decay', C.c_double)]
+  _fields_ = [('m', vp), ('v', vp), ('step', vp), ('lr', C.c_double), ('beta1', C.c_double), ('beta2', C.c_double), ('eps', C.c_double), ('weight_decay', C.c_double), ('lr_r', vp),
+              ('weight_decay_r', vp), ('replica_floats', C.c_int64)]
 
 
 class Batch(C.Structure):
@@ -44,7 +45,7 @@ class SacArgs(C.Structure):
   _fields_ = [('actor', Mlp), ('critic', Mlp), ('target', Mlp), ('actor_opt', Adam), ('critic_opt', Adam), ('alpha_opt', Adam), ('log_alpha', vp), ('batch', Batch),
               ('absorbing', vp), ('absorbing_from_state', C.c_int32), ('R', C.c_int32), ('eps_next', vp), ('eps_new', vp), ('discount', C.c_float),
               ('entropy_target', C.c_float), ('polyak_factor', C.c_float), ('_pad0', C.c_float), ('out_log_probs', vp), ('out_q_values', vp), ('out_losses', vp),
-              ('workspace', vp), ('workspace_bytes', C.c_int64)]
+              ('workspace', vp), ('workspace_bytes', C.c_int64), ('discount_r', vp), ('entropy_target_r', vp), ('polyak_r', vp)]
 
 
 class BcArgs(C.Structure):
@@ -58,18 +59,20 @@ class Gail(C.Structure):
 class GailUpdateArgs(C.Structure):
   _fields_ = [('disc', Gail), ('opt', Adam), ('policy', Batch), ('expert', Batch), ('eps_gp', vp), ('eps_mix', vp), ('R', C.c_int32), ('loss_function', C.c_int32),
               ('training', C.c_int32), ('_pad', C.c_int32), ('grad_penalty', C.c_float), ('entropy_bonus', C.c_float), ('pos_class_prior', C.c_float),
-              ('nonnegative_margin', C.c_float), ('out_losses', vp), ('workspace', vp), ('workspace_bytes', C.c_int64)]
+              ('nonnegative_margin', C.c_float), ('out_losses', vp), ('workspace', vp), ('workspace_bytes', C.c_int64), ('grad_penalty_r', vp), ('entropy_bonus_r', vp)]
 
 
 class Gailx(C.Structure):
   _fields_ = [('g', Mlp), ('h', Mlp), ('g_u', vp), ('g_v', vp), ('h_u', vp), ('h_v', vp), ('g_u_stride', C.c_int32), ('g_v_stride', C.c_int32), ('h_u_stride', C.c_int32),
-              ('h_v_stride', C.c_int32), ('state_only', C.c_int32), ('reward_function', C.c_int32), ('subtract_log_policy', C.c_int32), ('discount', C.c_float)]
+              ('h_v_stride', C.c_int32), ('state_only', C.c_int32), ('reward_function', C.c_int32), ('subtract_log_policy', C.c_int32), ('discount', C.c_float),
+              ('discount_r', vp)]
 
 
 class GailxUpdateArgs(C.Structure):
   _fields_ = [('disc', Gailx), ('opt', Adam), ('params_floats', C.c_int64), ('policy', Batch), ('expert', Batch), ('eps_gp', vp), ('eps_mix', vp), ('logp_policy', vp),
               ('logp_expert', vp), ('logp_mix', vp), ('R', C.c_int32), ('loss_function', C.c_int32), ('training', C.c_int32), ('_pad', C.c_int32), ('grad_penalty', C.c_float),
-              ('entropy_bonus', C.c_float), ('pos_class_prior', C.c_float), ('nonnegative_margin', C.c_float), ('out_losses', vp), ('workspace', vp), ('workspace_bytes', C.c_int64)]
+              ('entropy_bonus', C.c_float), ('pos_class_prior', C.c_float), ('nonnegative_margin', C.c_float), ('out_losses', vp), ('workspace', vp), ('workspace_bytes', C.c_int64),
+              ('grad_penalty_r', vp), ('entropy_bonus_r', vp)]
 
 
 class Red(C.Structure):
@@ -83,7 +86,8 @@ class RedUpdateArgs(C.Structure):
 
 class Pwil(C.Structure):
   _fields_ = [('atoms', vp), ('scale', vp), ('offset', vp), ('weights', vp), ('N', C.c_int32), ('d', C.c_int32), ('S', C.c_int32), ('A', C.c_int32), ('state_only', C.c_int32),
-              ('time_horizon', C.c_int32), ('reward_scale', C.c_float), ('reward_bandwidth', C.c_float)]
+              ('time_horizon', C.c_int32), ('reward_scale', C.c_float), ('reward_bandwidth', C.c_float),
+              ('reward_scale_r', vp), ('reward_bandwidth_r', vp)]
 
 
 class Env(C.Structure):

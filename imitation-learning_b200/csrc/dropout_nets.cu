@@ -276,7 +276,9 @@ extern "C" int il_red_update(il_handle* h, const il_red_update_args* a, void* st
   IL_CUDA(cudaMemsetAsync(w.grads, 0, (size_t)R * d->predictor.stride * 4, st));
   const MatView X = mk.in ? MatView{w.xin, (int64_t)B * din, 1, din} : MatView{a->batch.rows, a->batch.replica_stride, 1, a->batch.row};
   IL_TRY(mlp_backward_dropout(h, &d->predictor, R, B, X, mk, w.pacts, MatView{w.dpred, (int64_t)B * din, 1, din}, w.grads, d->predictor.stride, w.tmpA, w.tmpB, st));
-  return launch_adam(h, d->predictor.params, w.grads, &a->opt, (int64_t)R * d->predictor.stride, st);
+  il_adam opt = a->opt;
+  opt.replica_floats = d->predictor.stride;
+  return launch_adam(h, d->predictor.params, w.grads, &opt, (int64_t)R * d->predictor.stride, st);
 }
 
 extern "C" int il_red_sigma(il_handle* h, const il_red* d, int R, const il_batch* batch, const float* mask_in, const float* const* mask_hid, void* workspace, int64_t workspace_bytes,
@@ -384,5 +386,7 @@ extern "C" int il_bc_update_dropout(il_handle* h, const il_bc_args* a, const flo
   if (a->out_loss) IL_TRY(bc_row_mean_launch(h, w.row_loss, a->out_loss, R, B, st));
   IL_CUDA(cudaMemsetAsync(w.grads, 0, (size_t)R * a->actor.stride * 4, st));
   IL_TRY(mlp_backward_dropout(h, &a->actor, R, B, X, mk, w.acts, MatView{w.dhead, (int64_t)B * out, 1, out}, w.grads, a->actor.stride, w.tmpA, w.tmpB, st));
-  return launch_adam(h, a->actor.params, w.grads, &a->opt, (int64_t)R * a->actor.stride, st);
+  il_adam opt = a->opt;
+  opt.replica_floats = a->actor.stride;
+  return launch_adam(h, a->actor.params, w.grads, &opt, (int64_t)R * a->actor.stride, st);
 }

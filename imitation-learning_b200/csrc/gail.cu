@@ -168,6 +168,9 @@ __global__ void __launch_bounds__(THREADS) gail_update_kernel(const GailUpdParam
   const float* eps_gp = a.eps_gp ? a.eps_gp + (int64_t)r * B : nullptr;
   const float* eps_mix = a.eps_mix ? a.eps_mix + (int64_t)r * B : nullptr;
   const float invB = 1.f / (float)B;
+  // this replica's hyperparameters (per-replica arrays, else the scalars); the gradient-penalty pass runs where grad_penalty > 0
+  const float grad_penalty = a.grad_penalty_r ? a.grad_penalty_r[r] : a.grad_penalty, entropy_bonus = a.entropy_bonus_r ? a.entropy_bonus_r[r] : a.entropy_bonus;
+  const double lr = a.opt.lr_r ? a.opt.lr_r[r] : a.opt.lr, wd = a.opt.weight_decay_r ? a.opt.weight_decay_r[r] : a.opt.weight_decay;
 
   // ---- load parameters / buffers -------------------------------------------------------------------------
   for (int i = tid; i < H * d; i += THREADS) { s.W1[i] = prm[p.off_w1 + i]; s.G1[i] = 0.f; }
@@ -186,7 +189,7 @@ __global__ void __launch_bounds__(THREADS) gail_update_kernel(const GailUpdParam
   int gp_pass = -1;
   if (a.loss_function == IL_LOSS_MIXUP) { kinds[n_pass] = PASS_MIX; pass_eps[n_pass++] = eps_mix; }
   else { kinds[n_pass++] = PASS_POLICY; kinds[n_pass++] = PASS_EXPERT; }
-  if (a.grad_penalty > 0.f) { gp_pass = n_pass; kinds[n_pass] = PASS_MIX; pass_eps[n_pass++] = eps_gp; }
+  if (grad_penalty > 0.f) { gp_pass = n_pass; kinds[n_pass] = PASS_MIX; pass_eps[n_pass++] = eps_gp; }
 
   // ---- phase 1: one power iteration per layer per train-mode forward; remember (u, v, sigma) of each ------
   const int SF = gail_slot_floats(H, d);
@@ -279,7 +282,7 @@ __global__ void __launch_bounds__(THREADS) gail_update_kernel(const GailUpdParam
             df = kind == PASS_EXPERT ? pr * w * (sg - 1.f) * invB + pu_gate * pr * w * sg * invB : -pu_gate * w * sg * invB;
             loss_part += kind == PASS_EXPERT ? pr * w * softplusf(-f) + pu_gate * pr * w * softplusf(f) : -pu_gate * w * softplusf(f);
           }
-          if (a.entropy_bonus > 0.f) df += a.entropy_bonus * w * f * sg * (1.f - sg) * invB;  // training.py:130-132
+          if (entropy_bonus > 0.f) df += entropy_bonus * w * f * sg * (1.f - sg) * invB;  // training.py:130-132
           s.DF[b] = df;
           gb2k += df;
         }
@@ -337,8 +340,8 @@ __global__ void __launch_bounds__(THREADS) gail_update_kernel(const GailUpdParam
           float pen = 0.f;
           for (int j = 0; j < d; ++j) pen = fmaf(s.GX[b * g.ldx + j], s.GX[b * g.ldx + j], pen);
           const float wm = s.CO[b];
-          loss_part += a.grad_penalty * wm * pen;
-          s.DF[b] = 2.f * a.grad_penalty * wm * invB;  // coef_b
+          loss_part += grad_penalty * wm * pen;
+          s.DF[b] = 2.f * grad_penalty * wm * invB;  // coef_b
         }
         __syncthreads();
         // dL/dw2e[h] += sum_b coef_b m[b,h] (W1e g_b)[h]
@@ -414,14 +417,14 @@ __global__ void __launch_bounds__(THREADS) gail_update_kernel(const GailUpdParam
   // ---- AdamW (train.py:84; torch _single_tensor_adam) -----------------------------------------------------------
   if (tid == 0) {
     const double t = (double)*a.opt.step;
-    s.scal[0] = (float)(a.opt.lr / (1.0 - pow(a.opt.beta1, t)));
+    s.scal[0] = (float)(lr / (1.0 - pow(a.opt.beta1, t)));
     s.scal[1] = (float)sqrt(1.0 - pow(a.opt.beta2, t));
   }
   __syncthreads();
   const float step_size = s.scal[0], bc2_sqrt = s.scal[1];
-  const float decay = (float)(1.0 - a.opt.lr * a.opt.weight_decay), w1 = (float)(1.0 - a.opt.beta1), w2c = (float)(1.0 - a.opt.beta2), beta2 = (float)a.opt.beta2,
+  const float decay = (float)(1.0 - lr * wd), w1 = (float)(1.0 - a.opt.beta1), w2c = (float)(1.0 - a.opt.beta2), beta2 = (float)a.opt.beta2,
               eps = (float)a.opt.eps;
-  const bool has_wd = a.opt.weight_decay != 0.0;
+  const bool has_wd = wd != 0.0;
   float* am = a.opt.m + (int64_t)r * a.disc.g.stride;
   float* avv = a.opt.v + (int64_t)r * a.disc.g.stride;
   auto adam = [&](int64_t off, float grad) {
@@ -601,6 +604,9 @@ __global__ void __launch_bounds__(THREADS, 2) gail_update_tiled_kernel(const Gai
   const float* eps_gp = a.eps_gp ? a.eps_gp + (int64_t)r * B : nullptr;
   const float* eps_mix = a.eps_mix ? a.eps_mix + (int64_t)r * B : nullptr;
   const float invB = 1.f / (float)B;
+  // this replica's hyperparameters (per-replica arrays, else the scalars); the gradient-penalty pass runs where grad_penalty > 0
+  const float grad_penalty = a.grad_penalty_r ? a.grad_penalty_r[r] : a.grad_penalty, entropy_bonus = a.entropy_bonus_r ? a.entropy_bonus_r[r] : a.entropy_bonus;
+  const double lr = a.opt.lr_r ? a.opt.lr_r[r] : a.opt.lr, wd = a.opt.weight_decay_r ? a.opt.weight_decay_r[r] : a.opt.weight_decay;
 
   for (int i = tid; i < H * d; i += THREADS) { s.W1[i] = prm[p.off_w1 + i]; s.G1[i] = 0.f; }
   for (int h = tid; h < H; h += THREADS) {
@@ -617,7 +623,7 @@ __global__ void __launch_bounds__(THREADS, 2) gail_update_tiled_kernel(const Gai
   int gp_pass = -1;
   if (a.loss_function == IL_LOSS_MIXUP) { kinds[n_pass] = PASS_MIX; pass_eps[n_pass++] = eps_mix; }
   else { kinds[n_pass++] = PASS_POLICY; kinds[n_pass++] = PASS_EXPERT; }
-  if (a.grad_penalty > 0.f) { gp_pass = n_pass; kinds[n_pass] = PASS_MIX; pass_eps[n_pass++] = eps_gp; }
+  if (grad_penalty > 0.f) { gp_pass = n_pass; kinds[n_pass] = PASS_MIX; pass_eps[n_pass++] = eps_gp; }
 
   // ---- phase 1: power iterations (identical to gail_update_kernel) -------------------------------------------------------------
   const int SF = gail_slot_floats(H, d);
@@ -745,7 +751,7 @@ __global__ void __launch_bounds__(THREADS, 2) gail_update_tiled_kernel(const Gai
               df = kind == PASS_EXPERT ? pr * w * (sg - 1.f) * invB + pu_gate * pr * w * sg * invB : -pu_gate * w * sg * invB;
               loss_part += kind == PASS_EXPERT ? pr * w * softplusf(-f) + pu_gate * pr * w * softplusf(f) : -pu_gate * w * softplusf(f);
             }
-            if (a.entropy_bonus > 0.f) df += a.entropy_bonus * w * f * sg * (1.f - sg) * invB;
+            if (entropy_bonus > 0.f) df += entropy_bonus * w * f * sg * (1.f - sg) * invB;
             gb2k += df;
           }
           s.DF[b] = df;  // padded rows: 0
@@ -816,8 +822,8 @@ __global__ void __launch_bounds__(THREADS, 2) gail_update_tiled_kernel(const Gai
             float pen = 0.f;
             for (int j = 0; j < d; ++j) pen = fmaf(s.GX[b * DP + j], s.GX[b * DP + j], pen);
             const float wmix = s.CO[b];
-            loss_part += a.grad_penalty * wmix * pen;
-            coef = 2.f * a.grad_penalty * wmix * invB;
+            loss_part += grad_penalty * wmix * pen;
+            coef = 2.f * grad_penalty * wmix * invB;
           }
           s.DF[b] = coef;
         }
@@ -894,14 +900,14 @@ __global__ void __launch_bounds__(THREADS, 2) gail_update_tiled_kernel(const Gai
   // ---- AdamW (train.py:84; torch _single_tensor_adam) -----------------------------------------------------------
   if (tid == 0) {
     const double t = (double)*a.opt.step;
-    s.scal[0] = (float)(a.opt.lr / (1.0 - pow(a.opt.beta1, t)));
+    s.scal[0] = (float)(lr / (1.0 - pow(a.opt.beta1, t)));
     s.scal[1] = (float)sqrt(1.0 - pow(a.opt.beta2, t));
   }
   __syncthreads();
   const float step_size = s.scal[0], bc2_sqrt = s.scal[1];
-  const float decay = (float)(1.0 - a.opt.lr * a.opt.weight_decay), w1c = (float)(1.0 - a.opt.beta1), w2c = (float)(1.0 - a.opt.beta2), beta2 = (float)a.opt.beta2,
+  const float decay = (float)(1.0 - lr * wd), w1c = (float)(1.0 - a.opt.beta1), w2c = (float)(1.0 - a.opt.beta2), beta2 = (float)a.opt.beta2,
               eps = (float)a.opt.eps;
-  const bool has_wd = a.opt.weight_decay != 0.0;
+  const bool has_wd = wd != 0.0;
   float* am = a.opt.m + (int64_t)r * a.disc.g.stride;
   float* avv = a.opt.v + (int64_t)r * a.disc.g.stride;
   auto adam = [&](int64_t off, float grad) {
@@ -1066,7 +1072,7 @@ extern "C" int il_gail_update(il_handle* h, const il_gail_update_args* a, void* 
   IL_CHECK(a->policy.row == row_layout(a->policy.S, a->policy.A).len && a->expert.row == a->policy.row, "il_gail_update: bad row length");
   IL_CHECK(a->opt.m && a->opt.v && a->opt.step, "il_gail_update: null optimiser state");
   IL_CHECK(a->loss_function >= 0 && a->loss_function <= 2, "il_gail_update: bad loss function %d", a->loss_function);
-  IL_CHECK(!(a->grad_penalty > 0.f && !a->eps_gp), "il_gail_update: grad_penalty > 0 needs eps_gp");
+  IL_CHECK(!((a->grad_penalty > 0.f || a->grad_penalty_r) && !a->eps_gp), "il_gail_update: grad_penalty > 0 (or grad_penalty_r) needs eps_gp");
   IL_CHECK(!(a->loss_function == IL_LOSS_MIXUP && !a->eps_mix), "il_gail_update: Mixup needs eps_mix");
   GailUpdParams p;
   p.a = *a;

@@ -171,6 +171,8 @@ struct LossParams {
   int n_pass, B, row, off_terminal, off_weight, loss_function, shaping;
   float discount, entropy_bonus, pos_class_prior, nonnegative_margin;
   float* out_losses;     // [R, 2]
+  const float* discount_r;       // [R] or nullptr (il_gailx.discount_r)
+  const float* entropy_bonus_r;  // [R] or nullptr
 };
 __device__ __forceinline__ float pass_logit(const PassView& v, const LossParams& p, int r, int b, float* one_minus_t) {
   const int64_t i = (int64_t)r * p.B + b;
@@ -178,7 +180,8 @@ __device__ __forceinline__ float pass_logit(const PassView& v, const LossParams&
   float omt = 1.f;
   if (p.shaping) {
     omt = 1.f - v.rows[(int64_t)r * v.rs + (int64_t)b * p.row + p.off_terminal];
-    f = f + omt * (p.discount * v.ohn[i] - v.ohs[i]);  // models.py:174
+    const float discount = p.discount_r ? p.discount_r[r] : p.discount;
+    f = f + omt * (discount * v.ohn[i] - v.ohs[i]);  // models.py:174
   }
   if (v.logp) f = f - v.logp[i];                      // models.py:175
   *one_minus_t = omt;
@@ -189,6 +192,7 @@ __global__ void __launch_bounds__(256) gailx_loss_kernel(const LossParams p) {
   __shared__ float red[32];
   const int r = blockIdx.x, B = p.B;
   const float invB = 1.f / (float)B;
+  const float discount = p.discount_r ? p.discount_r[r] : p.discount, entropy_bonus = p.entropy_bonus_r ? p.entropy_bonus_r[r] : p.entropy_bonus;
   float pu_gate = 1.f;
   if (p.loss_function == IL_LOSS_PUGAIL) {  // the clamp of training.py:102 needs the batch scalar first
     float sp = 0.f, se = 0.f;
@@ -222,10 +226,10 @@ __global__ void __launch_bounds__(256) gailx_loss_kernel(const LossParams p) {
         df = v.kind == 1 ? pr * w * (sg - 1.f) * invB + pu_gate * pr * w * sg * invB : -pu_gate * w * sg * invB;
         loss += v.kind == 1 ? pr * w * softplusf(-f) + pu_gate * pr * w * softplusf(f) : -pu_gate * w * softplusf(f);
       }
-      if (p.entropy_bonus > 0.f) df += p.entropy_bonus * w * f * sg * (1.f - sg) * invB;
+      if (entropy_bonus > 0.f) df += entropy_bonus * w * f * sg * (1.f - sg) * invB;
       const int64_t i = (int64_t)r * B + b;
       v.dg[i] = df;
-      if (p.shaping) { v.dhn[i] = df * omt * p.discount; v.dhs[i] = -df * omt; }
+      if (p.shaping) { v.dhn[i] = df * omt * discount; v.dhs[i] = -df * omt; }
     }
   }
   loss = block_sum(loss, red);
@@ -269,9 +273,10 @@ __global__ void gp_linear_gx_kernel(const float* __restrict__ w1, int64_t w_gs, 
 }
 // P_b = lambda w_b |g_in|^2;  gbar = 2 lambda w_b / B * g_in (in place);  loss = mean(P). One CTA per replica.
 __global__ void __launch_bounds__(256) gp_penalty_kernel(float* __restrict__ gin, int ld, int cols, const float* __restrict__ rows, int64_t rs, int row, int off_weight, float lambda,
-                                                         float* __restrict__ out_losses, int B) {
+                                                         const float* __restrict__ lambda_r, float* __restrict__ out_losses, int B) {
   __shared__ float red[32];
   const int r = blockIdx.x;
+  if (lambda_r) lambda = lambda_r[r];
   float loss = 0.f;
   for (int b = threadIdx.x; b < B; b += blockDim.x) {
     float* g = gin + ((int64_t)r * B + b) * ld;
@@ -614,6 +619,7 @@ extern "C" int il_gailx_update(il_handle* h, const il_gailx_update_args* a, void
   LossParams lp{};
   lp.n_pass = n_loss_pass; lp.B = B; lp.row = row; lp.off_terminal = RL.terminal; lp.off_weight = RL.weight; lp.loss_function = a->loss_function; lp.shaping = shaping;
   lp.discount = d.discount; lp.entropy_bonus = a->entropy_bonus; lp.pos_class_prior = a->pos_class_prior; lp.nonnegative_margin = a->nonnegative_margin; lp.out_losses = a->out_losses;
+  lp.discount_r = d.discount_r; lp.entropy_bonus_r = a->entropy_bonus_r;
   for (int k = 0; k < n_loss_pass; ++k) {
     PassView& v = lp.pass[k];
     NetEval* e = &L.ev[k * per_pass];
@@ -645,7 +651,8 @@ extern "C" int il_gailx_update(il_handle* h, const il_gailx_update_args* a, void
     // keep for the double backward: with reward shaping g is linear (no chain) and h owns the scratch; without shaping there is only g.
     IL_TRY(gp_input_gradient(h, e[0], one, L.gb, L.gin, ld, 0, R, B, st));
     if (shaping) IL_TRY(gp_input_gradient(h, e[2], kh, L.gb, L.gin, ld, 1, R, B, st));
-    IL_LAUNCH(h, gp_penalty_kernel, R, 256, 0, st, L.gin, ld, ld, pass_rows[n_loss_pass], pass_rs[n_loss_pass], row, RL.weight, a->grad_penalty, a->out_losses, B);
+    IL_LAUNCH(h, gp_penalty_kernel, R, 256, 0, st, L.gin, ld, ld, pass_rows[n_loss_pass], pass_rs[n_loss_pass], row, RL.weight, a->grad_penalty, a->grad_penalty_r, a->out_losses,
+              B);
     GX_STAGE(h, st, "gp input gradients + penalty");
     if (shaping) {
       IL_TRY(gp_double_backward(h, e[2], kh, L.gb, L.gin, ld, R, B, st));
@@ -659,7 +666,9 @@ extern "C" int il_gailx_update(il_handle* h, const il_gailx_update_args* a, void
     GX_STAGE(h, st, "gp project g");
   }
   // ---- AdamW over the flat parameter buffer (train.py:84) ------------------------------------------------------------------------
-  return launch_adam(h, d.g.params, L.g_flat, &a->opt, a->params_floats, st);
+  il_adam opt = a->opt;
+  opt.replica_floats = pstride;
+  return launch_adam(h, d.g.params, L.g_flat, &opt, a->params_floats, st);
 }
 
 extern "C" int64_t il_gailx_reward_workspace_bytes(const il_gailx* d, int R, int B) {
@@ -694,7 +703,7 @@ extern "C" int il_gailx_reward(il_handle* h, const il_gailx* d, int R, const il_
     IL_TRY(eval_forward(h, ev[j], R, B, st));
   }
   LossParams lp{};
-  lp.B = B; lp.row = row; lp.off_terminal = RL.terminal; lp.off_weight = RL.weight; lp.shaping = shaping; lp.discount = d->discount;
+  lp.B = B; lp.row = row; lp.off_terminal = RL.terminal; lp.off_weight = RL.weight; lp.shaping = shaping; lp.discount = d->discount; lp.discount_r = d->discount_r;
   PassView v{};
   v.rows = batch->rows; v.rs = batch->replica_stride; v.og = ev[0].out;
   if (shaping) { v.ohn = ev[1].out; v.ohs = ev[2].out; }

@@ -204,7 +204,10 @@ __global__ void __launch_bounds__(256) pwil_reward_kernel(const il_pwil p, int R
     }
     __syncthreads();
   }
-  if (tid == 0) reward[r] = (float)((double)p.reward_scale * exp(-(double)p.reward_bandwidth * cost));  // models.py:249
+  if (tid == 0) {  // models.py:249
+    const float scale = p.reward_scale_r ? p.reward_scale_r[r] : p.reward_scale, bandwidth = p.reward_bandwidth_r ? p.reward_bandwidth_r[r] : p.reward_bandwidth;
+    reward[r] = (float)((double)scale * exp(-(double)bandwidth * cost));
+  }
 }
 
 __global__ void pwil_reset_kernel(float* __restrict__ weights, int N, int R, const int32_t* __restrict__ mask) {

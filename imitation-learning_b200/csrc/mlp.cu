@@ -406,8 +406,37 @@ __global__ void __launch_bounds__(256) mlp_small_forward_kernel(const SmallFwdAr
   }
 }
 
+// Per-replica hyperparameters of one AdamW launch (il_adam.lr_r / weight_decay_r, il_sac_args.polyak_r). The PR kernel variants build a
+// table of every replica's float step size, decay and polyak pair in shared memory once per CTA (the double expressions of the scalar path)
+// and look it up per 4-float chunk: replica_floats is a multiple of 4, so a chunk never straddles two replicas.
+struct AdamRep {
+  const double* lr;
+  const double* wd;
+  const float* tau;
+  int64_t rf;                         // floats per replica
+  double inv_rf;
+  int nrep;
+};
+constexpr int ADAM_MAX_REPLICAS = 4096; // shared-memory table: 16 B per replica
+__device__ __forceinline__ int adam_replica(int64_t i, const AdamRep& r) {  // i / rf without a 64-bit division
+  int64_t q = (int64_t)((double)i * r.inv_rf);
+  if (q * r.rf > i) --q;
+  else if ((q + 1) * r.rf <= i) ++q;
+  return (int)q;
+}
+__device__ __forceinline__ void adam_fill_table(float4* tab, const AdamRep& r, double bc1, double lr, double wd, float tau) {
+  for (int k = threadIdx.x; k < r.nrep; k += blockDim.x) {
+    const double l = r.lr ? r.lr[k] : lr, w = r.wd ? r.wd[k] : wd;
+    const float t = r.tau ? r.tau[k] : tau;
+    tab[k] = make_float4((float)(l / bc1), (float)(1.0 - l * w), t, (float)(1.0 - (double)t));
+  }
+}
+
+template <bool PR>
 __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, const int64_t* __restrict__ step,
-                            double lr, double beta1_d, double beta2_d, double eps_d, double wd, int64_t n, float* __restrict__ target, float tau, float one_minus_tau) {
+                            double lr, double beta1_d, double beta2_d, double eps_d, double wd, int64_t n, float* __restrict__ target, float tau, float one_minus_tau,
+                            const AdamRep rep) {
+  extern __shared__ float4 adam_tab[];  // PR: [nrep] (step size, decay, tau, 1 - tau)
   __shared__ float s_step_size, s_bc2_sqrt;
   if (threadIdx.x == 0) {  // torch _single_tensor_adam: Python-double scalars, then cast to the tensor dtype
     const double t = (double)*step;
@@ -415,11 +444,12 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
     s_step_size = (float)(lr / bc1);
     s_bc2_sqrt = (float)sqrt(bc2);
   }
+  if (PR) adam_fill_table(adam_tab, rep, 1.0 - pow(beta1_d, (double)*step), lr, wd, tau);
   __syncthreads();
-  const float step_size = s_step_size, bc2_sqrt = s_bc2_sqrt;
-  const float decay = (float)(1.0 - lr * wd), w1 = (float)(1.0 - beta1_d), w2 = (float)(1.0 - beta2_d);
+  float step_size = s_step_size, decay = (float)(1.0 - lr * wd);
+  const float bc2_sqrt = s_bc2_sqrt, w1 = (float)(1.0 - beta1_d), w2 = (float)(1.0 - beta2_d);
   const float beta2 = (float)beta2_d, eps = (float)eps_d;
-  const bool has_wd = wd != 0.0;
+  bool has_wd = wd != 0.0;
   auto upd = [&](float& pi, float& mi, float& vi, float gi) {
     if (has_wd) pi = __fmul_rn(pi, decay);                                     // param.mul_(1 - lr * weight_decay)
     mi = __fadd_rn(mi, __fmul_rn(w1, __fsub_rn(gi, mi)));                      // exp_avg.lerp_(grad, 1 - beta1)
@@ -427,9 +457,14 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
     const float denom = __fadd_rn(__fdiv_rn(sqrtf(vi), bc2_sqrt), eps);        // (exp_avg_sq.sqrt() / bias_correction2_sqrt).add_(eps)
     pi = __fadd_rn(pi, __fmul_rn(-step_size, __fdiv_rn(mi, denom)));           // param.addcdiv_(exp_avg, denom, value=-step_size)
   };
+  auto use_replica = [&](int64_t i) {  // decay == 1 is the scalar path's "weight_decay == 0": both leave the parameter unchanged
+    const float4 e = adam_tab[adam_replica(i, rep)];
+    step_size = e.x; decay = e.y; has_wd = e.y != 1.f; tau = e.z; one_minus_tau = e.w;
+  };
   // n is a multiple of 4 and all buffers are 16-byte aligned (flat parameter layout): 128-bit streams
   const int64_t n4 = n >> 2;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+    if (PR) use_replica(i << 2);
     float4 pv = reinterpret_cast<float4*>(p)[i], mv = reinterpret_cast<float4*>(m)[i], vv = reinterpret_cast<float4*>(v)[i];
     const float4 gv = reinterpret_cast<const float4*>(g)[i];
     upd(pv.x, mv.x, vv.x, gv.x); upd(pv.y, mv.y, vv.y, gv.y); upd(pv.z, mv.z, vv.z, gv.z); upd(pv.w, mv.w, vv.w, gv.w);
@@ -442,6 +477,7 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
     }
   }
   for (int64_t i = (n4 << 2) + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {  // tail (< 4 elements)
+    if (PR) use_replica(i);
     float pi = p[i], mi = m[i], vi = v[i];
     upd(pi, mi, vi, g[i]);
     p[i] = pi; m[i] = mi; v[i] = vi;
@@ -454,7 +490,7 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
 // the LSU only sees shared-memory traffic, global traffic is 128-byte-line bulk transfers on the copy engine path. Double buffered.
 constexpr int ADAM_STREAMS = 5;                 // p, g, m, v, target
 constexpr int ADAM_CONSUMERS = 256;             // threads 0..255 compute; warp 8 (one elected lane) drives the copy engine
-template <int TILE, int STAGES> constexpr int adam_tma_smem() { return STAGES * ADAM_STREAMS * TILE * 4 + 2 * STAGES * 8 + 64; }
+template <int TILE, int STAGES> constexpr int adam_tma_smem() { return STAGES * ADAM_STREAMS * TILE * 4 + 2 * STAGES * 8 + 64; }  // + 16 B per replica (PR)
 __device__ __forceinline__ void adam_mbar_wait(uint32_t bar, uint32_t parity) {
   asm volatile(
       "{\n\t.reg .pred q;\n\t"
@@ -467,10 +503,10 @@ __device__ __forceinline__ void adam_mbar_wait(uint32_t bar, uint32_t parity) {
 // TILE floats per operand per stage, STAGES-deep ring. Warp-specialised: the copy thread keeps STAGES - 1 tiles of loads in flight and turns
 // every computed stage into bulk stores; the 256 compute threads only ever wait on "stage full" and signal "stage computed" (no CTA-wide barrier
 // in the loop).
-template <int TILE, int STAGES>
+template <int TILE, int STAGES, bool PR>
 __global__ void __launch_bounds__(ADAM_CONSUMERS + 32) adam_tma_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                                                                       const int64_t* __restrict__ step, double lr, double beta1_d, double beta2_d, double eps_d, double wd, int64_t n,
-                                                                      float* __restrict__ target, float tau, float one_minus_tau) {
+                                                                      float* __restrict__ target, float tau, float one_minus_tau, const AdamRep rep) {
   extern __shared__ __align__(128) uint8_t adam_smem[];
   float* buf = reinterpret_cast<float*>(adam_smem);                                  // [stage][stream][TILE]
   const uint32_t smem0 = (uint32_t)__cvta_generic_to_shared(buf);
@@ -487,6 +523,8 @@ __global__ void __launch_bounds__(ADAM_CONSUMERS + 32) adam_tma_kernel(float* __
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
+  float4* tab = reinterpret_cast<float4*>(adam_smem + adam_tma_smem<TILE, STAGES>());  // PR: [nrep] behind the ring and the barriers
+  if (PR) adam_fill_table(tab, rep, 1.0 - pow(beta1_d, (double)*step), lr, wd, tau);
   __syncthreads();
   const int64_t n_tiles = (n + TILE - 1) / TILE;
   const int n_streams = target ? 5 : 4;
@@ -526,9 +564,9 @@ __global__ void __launch_bounds__(ADAM_CONSUMERS + 32) adam_tma_kernel(float* __
     return;
   }
   // ---- compute threads ----
-  const float step_size = s_step_size, bc2_sqrt = s_bc2_sqrt;
-  const float decay = (float)(1.0 - lr * wd), w1 = (float)(1.0 - beta1_d), w2 = (float)(1.0 - beta2_d), beta2 = (float)beta2_d, eps = (float)eps_d;
-  const bool has_wd = wd != 0.0;
+  float step_size = s_step_size, decay = (float)(1.0 - lr * wd);
+  const float bc2_sqrt = s_bc2_sqrt, w1 = (float)(1.0 - beta1_d), w2 = (float)(1.0 - beta2_d), beta2 = (float)beta2_d, eps = (float)eps_d;
+  bool has_wd = wd != 0.0;
   auto upd = [&](float& pi, float& mi, float& vi, float gi) {
     if (has_wd) pi = __fmul_rn(pi, decay);
     mi = __fadd_rn(mi, __fmul_rn(w1, __fsub_rn(gi, mi)));
@@ -547,6 +585,10 @@ __global__ void __launch_bounds__(ADAM_CONSUMERS + 32) adam_tma_kernel(float* __
     float4* sv = reinterpret_cast<float4*>(buf + (stage * ADAM_STREAMS + 3) * TILE);
     float4* stg = reinterpret_cast<float4*>(buf + (stage * ADAM_STREAMS + 4) * TILE);
     for (int i = tid; i < nf4; i += ADAM_CONSUMERS) {
+      if (PR) {
+        const float4 e = tab[adam_replica(tile * TILE + 4 * i, rep)];
+        step_size = e.x; decay = e.y; has_wd = e.y != 1.f; tau = e.z; one_minus_tau = e.w;
+      }
       float4 pv = sp[i], mv = smm[i], vv = sv[i];
       const float4 gv = sg[i];
       upd(pv.x, mv.x, vv.x, gv.x); upd(pv.y, mv.y, vv.y, gv.y); upd(pv.z, mv.z, vv.z, gv.z); upd(pv.w, mv.w, vv.w, gv.w);
@@ -564,11 +606,18 @@ __global__ void __launch_bounds__(ADAM_CONSUMERS + 32) adam_tma_kernel(float* __
 }
 
 template <int TILE, int STAGES>
-static int launch_adam_tma(il_handle* h, int ctas_per_sm, float* params, const float* grads, const il_adam* opt, int64_t n, cudaStream_t stream, float* polyak_target, float polyak_factor) {
+static int launch_adam_tma(il_handle* h, int ctas_per_sm, float* params, const float* grads, const il_adam* opt, int64_t n, cudaStream_t stream, float* polyak_target, float polyak_factor,
+                           const AdamRep& rep) {
   static bool attr_set = false;
-  if (!attr_set) { IL_CUDA(cudaFuncSetAttribute(adam_tma_kernel<TILE, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, adam_tma_smem<TILE, STAGES>())); attr_set = true; }
-  IL_LAUNCH(h, (adam_tma_kernel<TILE, STAGES>), h->sm_count * ctas_per_sm, ADAM_CONSUMERS + 32, (adam_tma_smem<TILE, STAGES>()), stream, params, grads, opt->m, opt->v, opt->step, opt->lr, opt->beta1,
-            opt->beta2, opt->eps, opt->weight_decay, n, polyak_target, polyak_factor, (float)(1.0 - (double)polyak_factor));
+  if (!attr_set) {
+    IL_CUDA(cudaFuncSetAttribute(adam_tma_kernel<TILE, STAGES, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, adam_tma_smem<TILE, STAGES>()));
+    IL_CUDA(cudaFuncSetAttribute(adam_tma_kernel<TILE, STAGES, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, adam_tma_smem<TILE, STAGES>() + 16 * ADAM_MAX_REPLICAS));
+    attr_set = true;
+  }
+  if (rep.nrep) IL_LAUNCH(h, (adam_tma_kernel<TILE, STAGES, true>), h->sm_count * ctas_per_sm, ADAM_CONSUMERS + 32, (size_t)(adam_tma_smem<TILE, STAGES>() + 16 * rep.nrep), stream, params, grads,
+                          opt->m, opt->v, opt->step, opt->lr, opt->beta1, opt->beta2, opt->eps, opt->weight_decay, n, polyak_target, polyak_factor, (float)(1.0 - (double)polyak_factor), rep);
+  else IL_LAUNCH(h, (adam_tma_kernel<TILE, STAGES, false>), h->sm_count * ctas_per_sm, ADAM_CONSUMERS + 32, (adam_tma_smem<TILE, STAGES>()), stream, params, grads, opt->m, opt->v, opt->step, opt->lr,
+                 opt->beta1, opt->beta2, opt->eps, opt->weight_decay, n, polyak_target, polyak_factor, (float)(1.0 - (double)polyak_factor), rep);
   return 0;
 }
 constexpr int ADAM_TMA_MIN_TILES = 4096;        // floats per CTA-iteration below which the plain kernel is used
@@ -714,27 +763,42 @@ int launch_actor_head(il_handle* h, const HeadFwdArgs& a, cudaStream_t stream) {
   return 0;
 }
 
-int launch_adam(il_handle* h, float* params, const float* grads, const il_adam* opt, int64_t n, cudaStream_t stream, float* polyak_target, float polyak_factor) {
+int launch_adam(il_handle* h, float* params, const float* grads, const il_adam* opt, int64_t n, cudaStream_t stream, float* polyak_target, float polyak_factor, const float* polyak_r) {
   IL_CHECK(opt->m && opt->v && opt->step, "adam: null state");
   IL_CHECK(((reinterpret_cast<uintptr_t>(params) | reinterpret_cast<uintptr_t>(grads) | reinterpret_cast<uintptr_t>(opt->m) | reinterpret_cast<uintptr_t>(opt->v) |
              reinterpret_cast<uintptr_t>(polyak_target)) & 15) == 0, "adam: buffers must be 16-byte aligned");
+  AdamRep rep{opt->lr_r, opt->weight_decay_r, polyak_target ? polyak_r : nullptr, opt->replica_floats, 0.0, 0};
+  if (rep.lr || rep.wd || rep.tau) {  // per-replica hyperparameters: the PR variants (the default step keeps the scalar kernels)
+    IL_CHECK(rep.rf > 0 && rep.rf % 4 == 0 && n % rep.rf == 0, "adam: per-replica hyperparameters need replica_floats (%lld) > 0, a multiple of 4 dividing n = %lld", (long long)rep.rf,
+             (long long)n);
+    rep.nrep = (int)(n / rep.rf);
+    rep.inv_rf = 1.0 / (double)rep.rf;
+    IL_CHECK(rep.nrep <= ADAM_MAX_REPLICAS, "adam: %d replicas with per-replica hyperparameters exceed %d", rep.nrep, ADAM_MAX_REPLICAS);
+  }
   if (h->adam_tma && n % 4 == 0 && n >= (int64_t)ADAM_TMA_MIN_TILES * h->sm_count * 2) {  // large flat buffers: TMA-staged streaming variant
     // Isolated launches on the bench buffers (profiles/r2_adam_variants.jsonl; copy = 6.5-6.6 TB/s): every geometry is within 8 % of the copy rate, the
     // 1-CTA-per-SM ones (4096 x 2, 2048 x 4) are the fastest alone (6.55 TB/s) — but inside the step the 2-CTA-per-SM 2048 x 2 ring wins (6.49 vs 6.59
     // ms / step, A/B in one gpurun call): its CTAs co-reside with the tail of the previous kernel and the head of the next.
     const int variant = h->adam_tma;
     switch (variant) {  // (tile floats, stages, CTAs per SM): 20 B/float of shared memory per stage
-      case 2: return launch_adam_tma<4096, 2>(h, 1, params, grads, opt, n, stream, polyak_target, polyak_factor);
-      case 3: return launch_adam_tma<2048, 3>(h, 1, params, grads, opt, n, stream, polyak_target, polyak_factor);
-      case 4: return launch_adam_tma<1024, 4>(h, 2, params, grads, opt, n, stream, polyak_target, polyak_factor);
-      case 5: return launch_adam_tma<1024, 3>(h, 3, params, grads, opt, n, stream, polyak_target, polyak_factor);
-      case 6: return launch_adam_tma<512, 4>(h, 4, params, grads, opt, n, stream, polyak_target, polyak_factor);
-      case 7: return launch_adam_tma<2048, 4>(h, 1, params, grads, opt, n, stream, polyak_target, polyak_factor);
-      default: return launch_adam_tma<2048, 2>(h, 2, params, grads, opt, n, stream, polyak_target, polyak_factor);
+      case 2: return launch_adam_tma<4096, 2>(h, 1, params, grads, opt, n, stream, polyak_target, polyak_factor, rep);
+      case 3: return launch_adam_tma<2048, 3>(h, 1, params, grads, opt, n, stream, polyak_target, polyak_factor, rep);
+      case 4: return launch_adam_tma<1024, 4>(h, 2, params, grads, opt, n, stream, polyak_target, polyak_factor, rep);
+      case 5: return launch_adam_tma<1024, 3>(h, 3, params, grads, opt, n, stream, polyak_target, polyak_factor, rep);
+      case 6: return launch_adam_tma<512, 4>(h, 4, params, grads, opt, n, stream, polyak_target, polyak_factor, rep);
+      case 7: return launch_adam_tma<2048, 4>(h, 1, params, grads, opt, n, stream, polyak_target, polyak_factor, rep);
+      default: return launch_adam_tma<2048, 2>(h, 2, params, grads, opt, n, stream, polyak_target, polyak_factor, rep);
     }
   }
-  IL_LAUNCH(h, adam_kernel, ew_blocks(n / 4 + 1, 256, h->sm_count), 256, 0, stream, params, grads, opt->m, opt->v, opt->step, opt->lr, opt->beta1, opt->beta2, opt->eps,
-            opt->weight_decay, n, polyak_target, polyak_factor, (float)(1.0 - (double)polyak_factor));
+  if (rep.nrep) {
+    static bool attr_set = false;
+    if (!attr_set) { IL_CUDA(cudaFuncSetAttribute(adam_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 16 * ADAM_MAX_REPLICAS)); attr_set = true; }
+    IL_LAUNCH(h, adam_kernel<true>, ew_blocks(n / 4 + 1, 256, h->sm_count), 256, (size_t)16 * rep.nrep, stream, params, grads, opt->m, opt->v, opt->step, opt->lr, opt->beta1, opt->beta2,
+              opt->eps, opt->weight_decay, n, polyak_target, polyak_factor, (float)(1.0 - (double)polyak_factor), rep);
+    return 0;
+  }
+  IL_LAUNCH(h, adam_kernel<false>, ew_blocks(n / 4 + 1, 256, h->sm_count), 256, 0, stream, params, grads, opt->m, opt->v, opt->step, opt->lr, opt->beta1, opt->beta2, opt->eps,
+            opt->weight_decay, n, polyak_target, polyak_factor, (float)(1.0 - (double)polyak_factor), rep);
   return 0;
 }
 

@@ -66,5 +66,7 @@ struct HeadFwdArgs {
 int launch_actor_head(il_handle* h, const HeadFwdArgs& a, cudaStream_t stream);
 
 // polyak_target != nullptr: also applies update_target_network (models.py:79-81) with the freshly stepped parameters
-int launch_adam(il_handle* h, float* params, const float* grads, const il_adam* opt, int64_t n, cudaStream_t stream, float* polyak_target = nullptr, float polyak_factor = 0.f);
+// polyak_r (nullable [R]): per-replica polyak factor, replica r = floats [r * opt->replica_floats, (r + 1) * opt->replica_floats)
+int launch_adam(il_handle* h, float* params, const float* grads, const il_adam* opt, int64_t n, cudaStream_t stream, float* polyak_target = nullptr, float polyak_factor = 0.f,
+                const float* polyak_r = nullptr);
 int launch_tick(il_handle* h, int64_t* s0, int64_t* s1, int64_t* s2, cudaStream_t stream);

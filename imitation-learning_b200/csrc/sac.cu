@@ -15,10 +15,12 @@ __device__ __forceinline__ float abs_at(const AbsView& v, int r, int b) { return
 
 // training.py:24-25: y = r + (1 - terminal) * discount * (min(Q1', Q2') - (1 - absorbing) * alpha * log_pi')
 __global__ void sac_target_kernel(const float* __restrict__ qt, const float* __restrict__ lp_next, const float* __restrict__ log_alpha, const float* __restrict__ rows,
-                                  int64_t rs, int row, int off_reward, int off_terminal, AbsView av, float discount, float* __restrict__ y, int R, int B) {
+                                  int64_t rs, int row, int off_reward, int off_terminal, AbsView av, float discount, const float* __restrict__ discount_r,
+                                  float* __restrict__ y, int R, int B) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (int64_t)R * B) return;
   const int r = (int)(i / B), b = (int)(i % B);
+  if (discount_r) discount = discount_r[r];
   const float alpha = expf(__ldg(log_alpha + r));
   const float* tr = rows + (int64_t)r * rs + (int64_t)b * row;
   const float q = fminf(qt[((int64_t)2 * r) * B + b], qt[((int64_t)2 * r + 1) * B + b]);
@@ -100,10 +102,14 @@ __global__ void sac_head_backward_kernel(const float* __restrict__ head, const f
 
 // training.py:45-49: temperature loss with the entry alpha, gradient w.r.t. log_alpha, Adam step (train.py:66). One block per replica.
 __global__ void sac_alpha_kernel(float* __restrict__ log_alpha, const float* __restrict__ lp_new, const float* __restrict__ rows, int64_t rs, int row, int off_weight,
-                                 AbsView av, float entropy_target, float* __restrict__ m, float* __restrict__ v, const int64_t* __restrict__ step, double lr,
-                                 double beta1, double beta2, double eps, double wd, float* __restrict__ out_losses, int B) {
+                                 AbsView av, float entropy_target, const float* __restrict__ entropy_target_r, float* __restrict__ m, float* __restrict__ v,
+                                 const int64_t* __restrict__ step, double lr, double beta1, double beta2, double eps, double wd, const double* __restrict__ lr_r,
+                                 const double* __restrict__ wd_r, float* __restrict__ out_losses, int B) {
   __shared__ float red[32];
   const int r = blockIdx.x;
+  if (entropy_target_r) entropy_target = entropy_target_r[r];
+  if (lr_r) lr = lr_r[r];
+  if (wd_r) wd = wd_r[r];
   float s = 0.f;
   for (int b = threadIdx.x; b < B; b += blockDim.x) {
     const float w = rows[(int64_t)r * rs + (int64_t)b * row + off_weight];
@@ -245,7 +251,7 @@ extern "C" int il_sac_update(il_handle* h, const il_sac_args* a, void* stream) {
   }
   // (2) target critics on (s', a') and the Bellman target  [training.py:24-25]
   IL_TRY(mlp_forward(h, &a->target, 2 * R, B, MatView{w.xn, (int64_t)B * d, 2, d}, w.critic_acts, w.q, (int64_t)B, 1, st, /*keep_hidden=*/false));
-  IL_LAUNCH(h, sac_target_kernel, ew, 128, 0, st, w.q, w.lp_next, a->log_alpha, rows, rs, row, L.reward, L.terminal, av, a->discount, w.y, R, B);
+  IL_LAUNCH(h, sac_target_kernel, ew, 128, 0, st, w.q, w.lp_next, a->log_alpha, rows, rs, row, L.reward, L.terminal, av, a->discount, a->discount_r, w.y, R, B);
   // (3) critic loss, backward, AdamW  [training.py:26-31]
   IL_TRY(mlp_forward(h, &a->critic, 2 * R, B, MatView{rows + L.state, rs, 2, row}, w.critic_acts, w.q, (int64_t)B, 1, st));
   IL_LAUNCH(h, sac_critic_lossgrad_kernel, R, 256, 0, st, w.q, w.y, rows, rs, row, L.weight, w.dq, a->out_q_values, a->out_losses, B);
@@ -253,7 +259,10 @@ extern "C" int il_sac_update(il_handle* h, const il_sac_args* a, void* stream) {
                       0, 0, 0, w.tmpA, w.tmpB, st));
   // polyak (training.py:52) is fused into the critic AdamW pass: the critic parameters do not change again inside this
   // update and the target is not read again, so the result equals the reference's end-of-update target step
-  IL_TRY(launch_adam(h, a->critic.params, w.g_critic, &a->critic_opt, (int64_t)2 * R * a->critic.stride, st, a->target.params, a->polyak_factor));
+  il_adam critic_opt = a->critic_opt, actor_opt = a->actor_opt;  // per-replica hyperparameters: replica r owns its twin (2 nets) / its actor
+  critic_opt.replica_floats = 2 * a->critic.stride;
+  actor_opt.replica_floats = a->actor.stride;
+  IL_TRY(launch_adam(h, a->critic.params, w.g_critic, &critic_opt, (int64_t)2 * R * a->critic.stride, st, a->target.params, a->polyak_factor, a->polyak_r));
   // (4) actor loss through the UPDATED critic  [training.py:34-42]
   IL_TRY(mlp_forward(h, &a->actor, R, B, MatView{rows + L.state, rs, 1, row}, w.actor_acts, w.head, (int64_t)B * 2 * A, 2 * A, st));
   {
@@ -274,10 +283,11 @@ extern "C" int il_sac_update(il_handle* h, const il_sac_args* a, void* stream) {
   IL_LAUNCH(h, sac_head_backward_kernel, ew, 128, 0, st, w.head, a->eps_new, w.xn, d, S, w.dxa, a->log_alpha, rows, rs, row, L.weight, av, w.dhead, R, B, A);
   IL_TRY(mlp_backward(h, &a->actor, R, B, MatView{rows + L.state, rs, 1, row}, w.actor_acts, MatView{w.dhead, (int64_t)B * 2 * A, 1, 2 * A}, w.g_actor, a->actor.stride,
                       nullptr, 0, 0, 0, 0, w.tmpA, w.tmpB, st));
-  IL_TRY(launch_adam(h, a->actor.params, w.g_actor, &a->actor_opt, (int64_t)R * a->actor.stride, st));
+  IL_TRY(launch_adam(h, a->actor.params, w.g_actor, &actor_opt, (int64_t)R * a->actor.stride, st));
   // (5) temperature  [training.py:45-49]
-  IL_LAUNCH(h, sac_alpha_kernel, R, 256, 0, st, a->log_alpha, lp_new, rows, rs, row, L.weight, av, a->entropy_target, a->alpha_opt.m, a->alpha_opt.v, a->alpha_opt.step,
-            a->alpha_opt.lr, a->alpha_opt.beta1, a->alpha_opt.beta2, a->alpha_opt.eps, a->alpha_opt.weight_decay, a->out_losses, B);
+  IL_LAUNCH(h, sac_alpha_kernel, R, 256, 0, st, a->log_alpha, lp_new, rows, rs, row, L.weight, av, a->entropy_target, a->entropy_target_r, a->alpha_opt.m, a->alpha_opt.v,
+            a->alpha_opt.step, a->alpha_opt.lr, a->alpha_opt.beta1, a->alpha_opt.beta2, a->alpha_opt.eps, a->alpha_opt.weight_decay, a->alpha_opt.lr_r, a->alpha_opt.weight_decay_r,
+            a->out_losses, B);
   return 0;  // (6) polyak [training.py:52]: done inside the critic AdamW kernel above
 }
 
@@ -335,5 +345,7 @@ extern "C" int il_bc_update(il_handle* h, const il_bc_args* a, void* stream) {
             a->out_loss ? w.row_loss : nullptr, R, B, A);
   if (a->out_loss) IL_LAUNCH(h, row_mean_kernel, R, 256, 0, st, w.row_loss, a->out_loss, B);
   IL_TRY(mlp_backward(h, &a->actor, R, B, X, w.acts, MatView{w.dhead, (int64_t)B * 2 * A, 1, 2 * A}, w.grads, a->actor.stride, nullptr, 0, 0, 0, 0, w.tmpA, w.tmpB, st));
-  return launch_adam(h, a->actor.params, w.grads, &a->opt, (int64_t)R * a->actor.stride, st);
+  il_adam opt = a->opt;
+  opt.replica_floats = a->actor.stride;
+  return launch_adam(h, a->actor.params, w.grads, &opt, (int64_t)R * a->actor.stride, st);
 }

@@ -16,6 +16,7 @@ from torch import Tensor
 from . import _lib
 from .memory import ReplayMemory, TransitionBatch
 from .net import ReplicaMLP, ReplicaRNG, init_fcnn_params, _null_ctx
+from .optim import per_replica
 
 
 def _cfg_get(cfg, key, default=None):
@@ -221,13 +222,18 @@ class SoftActor(_Module):
     _lib.check(_lib.lib().il_dril_reward(_lib.handle(), lp.data_ptr(), R, B, self.ENSEMBLE, None, 0, None, 0, 0, var.data_ptr(), _lib.stream()))
     return self._squeeze(var)
 
-  def set_uncertainty_threshold(self, expert_state: Tensor, expert_action: Tensor, quantile_cutoff: float, masks=None):  # :110-111 (one-off set-up statistic)
+  def set_uncertainty_threshold(self, expert_state: Tensor, expert_action: Tensor, quantile_cutoff, masks=None):  # :110-111 (one-off set-up statistic)
+    """quantile_cutoff: a float, or one cutoff per replica ([R]; each row's quantile is taken on the host side of the set-up, row by row)."""
     R = self.replicas
     es = torch.as_tensor(expert_state, dtype=torch.float32).to(self.device)
     ea = torch.as_tensor(expert_action, dtype=torch.float32).to(self.device)
     if es.dim() == 2: es, ea = es.unsqueeze(0).expand(R, -1, -1), ea.unsqueeze(0).expand(R, -1, -1)
     var = self._get_action_uncertainty(es, ea, masks=masks).reshape(R, -1)
-    self._q = torch.quantile(var, quantile_cutoff, dim=1).contiguous()
+    if isinstance(quantile_cutoff, (int, float)): self._q = torch.quantile(var, quantile_cutoff, dim=1).contiguous()
+    else:
+      cut = [float(c) for c in torch.as_tensor(quantile_cutoff).reshape(-1).tolist()]
+      assert len(cut) == R, f'{len(cut)} quantile cutoffs for {R} replicas'
+      self._q = torch.cat([torch.quantile(var[r:r + 1], cut[r], dim=1) for r in range(R)]).contiguous()
     self.q = float(self._q[0]) if R == 1 else self._q
 
   def predict_reward(self, state: Tensor, action: Tensor, masks=None, out: Optional[Tensor] = None) -> Tensor:  # :113-120
@@ -323,9 +329,11 @@ class GAILDiscriminator(_Module):
   """:152-180. Accelerated configuration: the depth-1 relu `g` network of conf/algorithm/GAIL.yaml (no reward
   shaping / log-policy subtraction), with or without spectral norm."""
 
-  def __init__(self, state_size: int, action_size: int, imitation_cfg, discount: float, replicas: int = 1, rng: Optional[ReplicaRNG] = None, device=None):
+  def __init__(self, state_size: int, action_size: int, imitation_cfg, discount, replicas: int = 1, rng: Optional[ReplicaRNG] = None, device=None):
+    """discount: a float, or one value per replica ([R]) for the reward-shaping term of the general discriminator."""
     model_cfg = imitation_cfg.discriminator
     self.discount, self.state_only = discount, bool(imitation_cfg.state_only)
+    self.discount_r = per_replica(discount, torch.device('cuda') if device is None else device)
     self.reward_shaping, self.subtract_log_policy, self.reward_function = bool(model_cfg.reward_shaping), bool(model_cfg.subtract_log_policy), model_cfg.reward_function
     self.state_size, self.action_size, self.replicas = state_size, action_size, replicas
     self.spectral_norm = bool(imitation_cfg.spectral_norm)
@@ -420,7 +428,9 @@ class GAILDiscriminator(_Module):
     if self.spectral_norm:
       d.g_u, d.g_v, d.g_u_stride, d.g_v_stride = self.g_u.data_ptr(), self.g_v.data_ptr(), self.g_u.stride(0), self.g_v.stride(0)
       if self.h_mlp is not None: d.h_u, d.h_v, d.h_u_stride, d.h_v_stride = self.h_u.data_ptr(), self.h_v.data_ptr(), self.h_u.stride(0), self.h_v.stride(0)
-    d.state_only, d.reward_function, d.subtract_log_policy, d.discount = int(self.state_only), _lib.REWARD[self.reward_function], int(self.subtract_log_policy), self.discount
+    d.state_only, d.reward_function, d.subtract_log_policy, d.discount = int(self.state_only), _lib.REWARD[self.reward_function], int(self.subtract_log_policy), \
+        0.0 if self.discount_r is not None else self.discount
+    d.discount_r = _lib.ptr(self.discount_r)
     return d
 
   def _general_state_items(self):
@@ -564,7 +574,9 @@ class GMMILDiscriminator:
 class PWILDiscriminator:
   """:216-249. The expert atoms are shared by all replicas; the remaining-weight vector is per replica."""
 
-  def __init__(self, state_size: int, action_size: int, imitation_cfg, expert_memory: ReplayMemory, time_horizon: int, replicas: int = 1, device=None):
+  def __init__(self, state_size: int, action_size: int, imitation_cfg, expert_memory: ReplayMemory, time_horizon: int, replicas: int = 1, device=None,
+               reward_scale=None, reward_bandwidth_scale=None):
+    """reward_scale / reward_bandwidth_scale override imitation_cfg's values with a float or one value per replica ([R])."""
     self.state_only, self.replicas = bool(imitation_cfg.state_only), replicas
     self.state_size, self.action_size, self.time_horizon = state_size, action_size, time_horizon
     self.expert_memory = expert_memory
@@ -574,8 +586,12 @@ class PWILDiscriminator:
     inv_scale[inv_scale == 0] = 1
     self.data_scale, self.data_offset = (1 / inv_scale).contiguous(), offset.contiguous()
     self.atoms = (self.data_scale * (atoms + self.data_offset)).contiguous()  # :229
-    self.reward_scale = imitation_cfg.reward_scale
-    self.reward_bandwidth = imitation_cfg.reward_bandwidth_scale * time_horizon / sqrt(state_size if self.state_only else state_size + action_size)  # :222
+    self.reward_scale = imitation_cfg.reward_scale if reward_scale is None else reward_scale
+    scale = imitation_cfg.reward_bandwidth_scale if reward_bandwidth_scale is None else reward_bandwidth_scale
+    if per_replica(scale, 'cpu') is not None: scale = per_replica(scale, 'cpu', torch.float64)  # the host expression below in double, replica by replica
+    self.reward_bandwidth = scale * time_horizon / sqrt(state_size if self.state_only else state_size + action_size)  # :222
+    self.reward_scale_r, self.reward_bandwidth_r = per_replica(self.reward_scale, self.device), per_replica(self.reward_bandwidth, self.device)
+    for t in (self.reward_scale_r, self.reward_bandwidth_r): assert t is None or t.numel() == replicas, 'one PWIL reward scale / bandwidth per replica'
     self.expert_weights = torch.empty(replicas, self.atoms.size(0), device=self.device)
     self.reset()
 
@@ -587,7 +603,10 @@ class PWILDiscriminator:
     p = _lib.Pwil()
     p.atoms, p.scale, p.offset, p.weights = self.atoms.data_ptr(), self.data_scale.data_ptr(), self.data_offset.data_ptr(), self.expert_weights.data_ptr()
     p.N, p.d, p.S, p.A = self.atoms.size(0), self.atoms.size(1), self.state_size, self.action_size
-    p.state_only, p.time_horizon, p.reward_scale, p.reward_bandwidth = int(self.state_only), self.time_horizon, self.reward_scale, self.reward_bandwidth
+    p.state_only, p.time_horizon = int(self.state_only), self.time_horizon
+    p.reward_scale = 0.0 if self.reward_scale_r is not None else self.reward_scale
+    p.reward_bandwidth = 0.0 if self.reward_bandwidth_r is not None else self.reward_bandwidth
+    p.reward_scale_r, p.reward_bandwidth_r = _lib.ptr(self.reward_scale_r), _lib.ptr(self.reward_bandwidth_r)
     return p
 
   def reset(self, mask: Optional[Tensor] = None):  # :228-230

@@ -17,7 +17,7 @@ import numpy as np
 import torch
 from torch import Tensor
 
-from . import _lib, distributed
+from . import _lib, distributed, sweep
 from .config import Config, load_config
 from .environments import D4RLEnv, ENVS
 from .evaluation import evaluate_agent
@@ -27,6 +27,7 @@ from .net import ReplicaRNG
 from .optim import Adam, AdamW
 
 ACCELERATED = ['AdRIL', 'BC', 'DRIL', 'SAC', 'GAIL', 'GMMIL', 'PWIL', 'RED']
+MAX_SWEEP_REPLICAS = 4096  # replicas per AdamW launch with per-replica hyperparameters (ADAM_MAX_REPLICAS, csrc/mlp.cu)
 
 
 def check_config(cfg: Config):
@@ -56,11 +57,16 @@ def check_config(cfg: Config):
 
 
 class Trainer:
-  def __init__(self, cfg: Config, replicas: Optional[int] = None, seed_offset: int = 0, fast_init: bool = False, device=None):
+  def __init__(self, cfg: Config, replicas: Optional[int] = None, seed_offset: int = 0, fast_init: bool = False, device=None, hparams: Optional[Dict[str, Tensor]] = None):
+    """hparams: {key: [R] values} of per-replica hyperparameters (the keys of sweep.BATCHABLE); replica r trains with its own values and
+    equals, bit for bit, a run configured with them. Without it every replica uses the config's values."""
     check_config(cfg)
     self.cfg = cfg
     self.R = R = int(cfg.get('replicas', 1) if replicas is None else replicas)
     self.device = dev = torch.device('cuda', torch.cuda.current_device()) if device is None else torch.device(device)
+    self.hparams = self._check_hparams(hparams or {}, cfg, R, dev)
+    hp = lambda key, default: self.hparams.get(key, default)  # float64 [R] (the optimisers keep lr / weight decay in double) or the config float
+    hp32 = lambda key, default: self.hparams[key].float() if key in self.hparams else default  # float scalars of the kernels, rounded like a Python float
     self.lib, self.h = _lib.lib(), _lib.handle(dev.index)
     _lib.check(self.lib.il_set_gemm_mode(self.h, _lib.GEMM_MODE[cfg.get('gemm_mode', 'fp32')]))
     self.seed = seed = cfg.seed + seed_offset
@@ -81,13 +87,16 @@ class Trainer:
     nrep = 1 if fast_init else R
     self.actor, self.critic = SoftActor(S, A, cfg.reinforcement.actor, replicas=nrep, rng=rng, device=dev), TwinCritic(S, A, cfg.reinforcement.critic, replicas=nrep, rng=rng, device=dev)
     self.discriminator = None
-    if self.algorithm == 'GAIL': self.discriminator = GAILDiscriminator(S, A, cfg.imitation, cfg.reinforcement.discount, replicas=nrep, rng=rng, device=dev)
+    self.discount, self.polyak = hp32('reinforcement.discount', cfg.reinforcement.discount), hp32('reinforcement.polyak_factor', cfg.reinforcement.polyak_factor)
+    if self.algorithm == 'GAIL': self.discriminator = GAILDiscriminator(S, A, cfg.imitation, self.discount, replicas=nrep, rng=rng, device=dev)
     elif self.algorithm == 'DRIL': self.discriminator = SoftActor(S, A, cfg.imitation.discriminator, replicas=nrep, rng=rng, device=dev)  # train.py:74
     elif self.algorithm == 'RED': self.discriminator = REDDiscriminator(S, A, cfg.imitation, replicas=nrep, rng=rng, device=dev)  # train.py:82
     if fast_init and R > 1: self._replicate()
     self.log_alpha = torch.zeros(R, device=dev)
-    self.target_critic, self.entropy_target = create_target_network(self.critic), cfg.reinforcement.target_temperature * A
-    lr, wd = cfg.training.learning_rate, cfg.training.weight_decay
+    self.target_critic = create_target_network(self.critic)
+    tt = hp('reinforcement.target_temperature', cfg.reinforcement.target_temperature)
+    self.entropy_target = (tt * A).float() if isinstance(tt, Tensor) else tt * A
+    lr, wd = hp('training.learning_rate', cfg.training.learning_rate), hp('training.weight_decay', cfg.training.weight_decay)
     self.actor_optimiser, self.critic_optimiser = AdamW(self.actor.parameters(), lr=lr, weight_decay=wd), AdamW(self.critic.parameters(), lr=lr, weight_decay=wd)
     self.temperature_optimiser = Adam([self.log_alpha], lr=lr)
     need = R * int(cfg.memory.size) * _lib.py_row_layout(S, A)[1] * 4
@@ -99,7 +108,8 @@ class Trainer:
     self.memory.seed = seed
     # train.py:70-84
     if self.algorithm in ('DRIL', 'GAIL', 'RED'):
-      self.discriminator_optimiser = AdamW(self.discriminator.parameters(), lr=cfg.imitation.learning_rate, weight_decay=cfg.imitation.weight_decay)  # train.py:83-84
+      self.discriminator_optimiser = AdamW(self.discriminator.parameters(), lr=hp('imitation.learning_rate', cfg.imitation.learning_rate),
+                                           weight_decay=hp('imitation.weight_decay', cfg.imitation.weight_decay))  # train.py:83-84
     if self.algorithm == 'GAIL':
       self.discriminator.eval()  # train.py:147
     elif self.algorithm == 'AdRIL':
@@ -108,7 +118,8 @@ class Trainer:
     elif self.algorithm == 'GMMIL':
       self.discriminator = GMMILDiscriminator(S, A, cfg.imitation, replicas=R, device=dev)
     elif self.algorithm == 'PWIL':
-      self.discriminator = PWILDiscriminator(S, A, cfg.imitation, self.expert_memory, self.env.max_episode_steps, replicas=R, device=dev)
+      self.discriminator = PWILDiscriminator(S, A, cfg.imitation, self.expert_memory, self.env.max_episode_steps, replicas=R, device=dev,
+                                             reward_scale=hp('imitation.reward_scale', None), reward_bandwidth_scale=hp('imitation.reward_bandwidth_scale', None))
     if self.expert_memory is not None: self.expert_memory.seed = seed + 7919
     if self.algorithm == 'PWIL' and cfg.imitation.mix_expert_data != 'none': self._pwil_relabel_expert()  # train.py:136-140
     if self.algorithm in ('GMMIL', 'PWIL') and cfg.imitation.mix_expert_data == 'prefill_memory': self.memory.transfer_transitions(self.expert_memory)  # train.py:141,143
@@ -131,6 +142,8 @@ class Trainer:
     self.sac_out = dict(log_probs=f(R, B), q_values=f(R, B), losses=f(R, 3))
     self.gail_losses = f(R, 2)
     self.rng = _RNG(seed, dev)
+    self.grad_penalty, self.entropy_bonus = hp32('imitation.grad_penalty', None), hp32('imitation.entropy_bonus', None)
+    self.grad_penalty_any = bool((self.hparams['imitation.grad_penalty'] > 0).any()) if 'imitation.grad_penalty' in self.hparams else None  # set-up time, never in a capture
     self.inject = False  # tests: True = all noise / index buffers are filled by the caller before each step
     self.dril_masks = None  # tests (inject): the dropout masks of this step's DRIL ensemble pass
     self.device_rng = bool(cfg.get('device_rng', True))
@@ -145,6 +158,25 @@ class Trainer:
                         entropies=[], Q_values=[])  # train.py:87
     self.score: List[float] = []
     self.env.batch.reset(self.env.reset_noise(R), self.state)  # train.py:146
+
+  @staticmethod
+  def _check_hparams(hparams, cfg: Config, R: int, dev) -> Dict[str, Tensor]:
+    if hparams and R > MAX_SWEEP_REPLICAS:
+      raise ValueError(f'per-replica hyperparameters support up to {MAX_SWEEP_REPLICAS} replicas per GPU (the per-replica AdamW kernels keep a table of every '
+                       f'replica in shared memory); {R} requested: use more GPUs or fewer replicas')
+    if cfg.algorithm == 'PWIL' and cfg.imitation.mix_expert_data != 'none' and {'imitation.reward_scale', 'imitation.reward_bandwidth_scale'} & set(hparams):
+      raise ValueError('PWIL reward scale / bandwidth cannot vary per replica with imitation.mix_expert_data != none: the expert memory shared by all replicas '
+                       'holds one relabelled reward per transition')
+    out = {}
+    for k, v in hparams.items():
+      if k not in sweep.BATCHABLE: raise ValueError(f'hparams: {k} cannot vary per replica; batchable keys: {", ".join(sweep.BATCHABLE)}')
+      t = torch.as_tensor(v, dtype=torch.float64).reshape(-1)
+      if t.numel() != R: raise ValueError(f'hparams: {k} has {t.numel()} values for {R} replicas')
+      host = t.cpu()
+      if k == 'imitation.quantile_cutoff' and not bool(((host >= 0) & (host <= 1)).all()): raise ValueError('hparams: quantile_cutoff outside [0, 1]')
+      if k in ('imitation.grad_penalty', 'imitation.entropy_bonus') and not bool((host >= 0).all()): raise ValueError(f'hparams: {k} must be >= 0')
+      out[k] = t.to(dev).contiguous()
+    return out
 
   def _pwil_relabel_expert(self):
     """train.py:136-140: the expert's own transitions get their greedy PWIL reward, walking the expert memory in order and
@@ -215,7 +247,8 @@ class Trainer:
       self.expert_memory.gather(self.idx_exp, out=self.expert_batch)
     if self.algorithm == 'GAIL':
       from .training import adversarial_imitation_update
-      if cfg.imitation.grad_penalty > 0 and not self.inject: self.rng.uniform(None, self.device, stream_id=5, out=self.eps_gp)
+      gp_draw = self.grad_penalty_any if self.grad_penalty is not None else cfg.imitation.grad_penalty > 0
+      if gp_draw and not self.inject: self.rng.uniform(None, self.device, stream_id=5, out=self.eps_gp)
       eps_mix = None
       if cfg.imitation.loss_function == 'Mixup':  # training.py:106: Beta(a, a) draws; a == 1 (all published configs) is U(0, 1)
         if float(cfg.imitation.mixup_alpha) != 1.0: raise NotImplementedError('mixup_alpha != 1 needs Beta draws; only mixup_alpha = 1 (the reference default) is on the graph-captured path')
@@ -223,7 +256,8 @@ class Trainer:
         eps_mix = self.eps_mix
       self.discriminator.train()  # train.py:178-180
       adversarial_imitation_update(self.actor, self.discriminator, self.batch, self.expert_batch, self.discriminator_optimiser, cfg.imitation, eps_gp=self.eps_gp,
-                                   eps_mix=eps_mix, out_losses=self.gail_losses)
+                                   eps_mix=eps_mix, out_losses=self.gail_losses, grad_penalty=self.grad_penalty, entropy_bonus=self.entropy_bonus,
+                                   grad_penalty_any=self.grad_penalty_any)
       self.discriminator.eval()
     if self.algorithm in ('GAIL', 'GMMIL'):
       if cfg.imitation.mix_expert_data == 'mixed_batch':
@@ -250,7 +284,7 @@ class Trainer:
       self.rng.normal(None, self.device, stream_id=6, out=self.eps_next)
       self.rng.normal(None, self.device, stream_id=7, out=self.eps_new)
     sac_update(self.actor, self.critic, self.log_alpha, self.target_critic, self.batch, self.actor_optimiser, self.critic_optimiser, self.temperature_optimiser,
-               cfg.reinforcement.discount, self.entropy_target, cfg.reinforcement.polyak_factor, eps_next=self.eps_next, eps_new=self.eps_new, out=self.sac_out)  # train.py:203
+               self.discount, self.entropy_target, self.polyak, eps_next=self.eps_next, eps_new=self.eps_new, out=self.sac_out)  # train.py:203
 
   def bc_pretrain(self, iterations: Optional[int] = None) -> Tensor:
     """train.py:93-99: `iterations` behavioural-cloning steps on epoch-wise shuffled expert minibatches (drop_last), with a
@@ -259,7 +293,8 @@ class Trainer:
     from .training import behavioural_cloning_update
     cfg, B, n = self.cfg, self.B, self.expert_memory.size
     iterations = cfg.bc_pretraining.iterations if iterations is None else iterations
-    opt = AdamW(self.actor.parameters(), lr=cfg.bc_pretraining.learning_rate, weight_decay=cfg.bc_pretraining.weight_decay)
+    opt = AdamW(self.actor.parameters(), lr=self.hparams.get('bc_pretraining.learning_rate', cfg.bc_pretraining.learning_rate),
+                weight_decay=self.hparams.get('bc_pretraining.weight_decay', cfg.bc_pretraining.weight_decay))
     loss = torch.zeros(self.R, device=self.device)
     per_epoch = max(n // B, 1)
     perm = None
@@ -291,7 +326,8 @@ class Trainer:
       else: target_estimation_update(d, self.expert_batch, self.discriminator_optimiser, masks=m)
     em = self.expert_memory
     if self.algorithm == 'DRIL':
-      d.set_uncertainty_threshold(em.rows[0, :, :self.S], em.rows[0, :, self.S:self.S + self.A], cfg.imitation.quantile_cutoff, masks=threshold_masks)  # train.py:127
+      d.set_uncertainty_threshold(em.rows[0, :, :self.S], em.rows[0, :, self.S:self.S + self.A], self.hparams.get('imitation.quantile_cutoff', cfg.imitation.quantile_cutoff),
+                                  masks=threshold_masks)  # train.py:127
     else:
       first = torch.arange(B, dtype=torch.int32, device=self.device).unsqueeze(0).expand(self.R, -1).contiguous() % n
       self.expert_memory.gather(first, out=self.expert_batch)
@@ -377,8 +413,19 @@ def train(cfg: Config, file_prefix: str = '') -> float:
   rank, world = distributed.init('nccl')
   total = int(cfg.get('replicas', 1))
   lo, hi = distributed.shard(total, rank, world)
-  trainer = Trainer(cfg, replicas=hi - lo, seed_offset=lo)
+  keys, values = sweep.setup(cfg)  # hyperparameter search on the replica axis (sweep.space / sweep.trials)
+  hparams, sweep_sums = None, []
+  if values is not None:
+    hparams = sweep.shard(sweep.replica_hparams(keys, values, total), lo, hi)
+    trials_here = sweep.trial_of(total, len(values))[lo:hi]
+  trainer = Trainer(cfg, replicas=hi - lo, seed_offset=lo, hparams=hparams)
   metrics, score = trainer.metrics, trainer.score
+
+  def sweep_eval(normalized):
+    if values is not None: sweep_sums.append(sweep.reduce_sums(sweep.trial_sums(normalized, trials_here, len(values))))
+
+  def sweep_save():
+    if values is not None and rank == 0: sweep.write_results(file_prefix, keys, values, total // len(values), sweep.scores(sweep_sums, len(values)))
   start_time = time.time()
   if cfg.bc_pretraining.iterations > 0:  # train.py:93-112
     trainer.bc_pretrain()
@@ -386,6 +433,8 @@ def train(cfg: Config, file_prefix: str = '') -> float:
       returns = trainer.evaluate()
       mean, std, n = distributed.return_statistics(returns)
       normalized = (returns.cpu().numpy() - trainer.normalization_min) / (trainer.normalization_max - trainer.normalization_min)
+      sweep_eval(normalized)
+      sweep_save()
       flat = total == 1
       metrics['test_steps'], metrics['test_returns'], metrics['test_returns_normalized'] = [0], [returns.cpu().numpy().reshape(-1).tolist() if flat else returns.cpu().numpy().tolist()], \
           [normalized.reshape(-1).tolist() if flat else normalized.tolist()]
@@ -403,6 +452,7 @@ def train(cfg: Config, file_prefix: str = '') -> float:
       mean, std, n = distributed.return_statistics(returns)
       normalized = (returns.cpu().numpy() - trainer.normalization_min) / (trainer.normalization_max - trainer.normalization_min)
       score.append(float((mean - trainer.normalization_min) / (trainer.normalization_max - trainer.normalization_min)))
+      sweep_eval(normalized)
       metrics['test_steps'].append(step)
       flat = total == 1  # the reference's schema: one list of `episodes` floats per evaluation (train.py:214-219); R > 1 keeps [R][episodes]
       metrics['test_returns'].append(returns.cpu().numpy().reshape(-1).tolist() if flat else returns.cpu().numpy().tolist())
@@ -419,6 +469,7 @@ def train(cfg: Config, file_prefix: str = '') -> float:
     torch.save(trainer.state_dicts(), f'{file_prefix}agent.pth')
     if cfg.algorithm in ('DRIL', 'GAIL', 'RED'): torch.save(trainer.discriminator.state_dict(), f'{file_prefix}discriminator.pth')  # train.py:238
     torch.save(metrics, f'{file_prefix}metrics.pth')
+  sweep_save()
   return float(np.mean(score)) if score else float('nan')
 
 

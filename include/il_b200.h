@@ -46,12 +46,20 @@ typedef struct il_mlp {
   int32_t _pad;
 } il_mlp;
 
-/* torch.optim.Adam / AdamW (decoupled decay) state over one flat parameter buffer (train.py:66,84). */
+/* torch.optim.Adam / AdamW (decoupled decay) state over one flat parameter buffer (train.py:66,84).
+ * Per-replica hyperparameters: lr_r / weight_decay_r (nullable [R] device arrays; NULL = the scalar for every replica) give replica r
+ * its own value, with the scalar path's arithmetic in double, so a replica equals a scalar run with its values bit for bit. Replica r
+ * owns floats [r * replica_floats, (r + 1) * replica_floats) of the buffer: il_adam_step / il_adam_step_polyak need replica_floats
+ * (a multiple of 4) when an array is set; the fused updates take it from their own layout. One call with per-replica values covers at
+ * most 4096 replicas (the AdamW kernels keep a 16-byte entry per replica in shared memory); more is an error. */
 typedef struct il_adam {
   float*   m;                       /* exp_avg, same shape as the parameter buffer */
   float*   v;                       /* exp_avg_sq */
   int64_t* step;                    /* device scalar, incremented by every update */
   double lr, beta1, beta2, eps, weight_decay;  /* Python floats in the reference; kept in double like torch does */
+  const double* lr_r;               /* [R] or NULL */
+  const double* weight_decay_r;     /* [R] or NULL */
+  int64_t replica_floats;           /* floats per replica (2 x stride for the twin critic) */
 } il_adam;
 
 /* Packed transitions [R, B, row]: row = [state S | action A | reward | next_state S | terminal | timeout |
@@ -150,6 +158,9 @@ typedef struct il_sac_args {
   float* out_losses;                /* [R, 3] value, policy, temperature loss (may be NULL) */
   void*   workspace;
   int64_t workspace_bytes;
+  const float* discount_r;          /* [R] per-replica discount / entropy_target / polyak_factor, or NULL = the scalar */
+  const float* entropy_target_r;
+  const float* polyak_r;
 } il_sac_args;
 int64_t il_sac_workspace_bytes(const il_sac_args* a);
 int il_sac_update(il_handle* h, const il_sac_args* a, void* stream);
@@ -264,6 +275,8 @@ typedef struct il_gail_update_args {
   float* out_losses;                /* [R, 2] bce/mixup loss, gp loss (may be NULL) */
   void*   workspace;                /* il_gail_workspace_bytes */
   int64_t workspace_bytes;
+  const float* grad_penalty_r;      /* [R] per-replica grad_penalty / entropy_bonus, or NULL = the scalar. grad_penalty_r needs eps_gp; */
+  const float* entropy_bonus_r;     /* the gradient-penalty pass runs for the replicas whose grad_penalty is > 0 */
 } il_gail_update_args;
 int64_t il_gail_workspace_bytes(const il_gail_update_args* a);
 /* adversarial_imitation_update (training.py:85-134) incl. the train()/eval() power-iteration semantics. */
@@ -286,6 +299,7 @@ typedef struct il_gailx {
   int32_t reward_function;          /* IL_REWARD_* */
   int32_t subtract_log_policy;      /* models.py:175 */
   float   discount;                 /* models.py:174 */
+  const float* discount_r;          /* [R] per-replica discount, or NULL = discount */
 } il_gailx;
 typedef struct il_gailx_update_args {
   il_gailx disc;
@@ -302,6 +316,8 @@ typedef struct il_gailx_update_args {
   float* out_losses;                /* [R, 2] (may be NULL) */
   void*   workspace;                /* il_gailx_workspace_bytes */
   int64_t workspace_bytes;
+  const float* grad_penalty_r;      /* [R] or NULL, as in il_gail_update_args. The scalar grad_penalty > 0 selects the gradient-penalty pass for */
+  const float* entropy_bonus_r;     /* every replica: one with grad_penalty_r[r] == 0 adds no penalty but still runs that pass's power iteration */
 } il_gailx_update_args;
 int64_t il_gailx_workspace_bytes(const il_gailx_update_args* a);
 int il_gailx_update(il_handle* h, const il_gailx_update_args* a, void* stream);      /* training.py:85-134 */
@@ -328,6 +344,8 @@ typedef struct il_pwil {
   int32_t  N, d, S, A;
   int32_t  state_only, time_horizon;
   float    reward_scale, reward_bandwidth;
+  const float* reward_scale_r;      /* [R] per-replica reward_scale / reward_bandwidth, or NULL = the scalar */
+  const float* reward_bandwidth_r;
 } il_pwil;
 int il_pwil_reset(il_handle* h, const il_pwil* p, int R, const int32_t* mask, void* stream);   /* models.py:228-230 */
 int il_pwil_reward(il_handle* h, const il_pwil* p, int R, const float* state, const float* action, float* reward,
