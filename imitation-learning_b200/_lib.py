@@ -123,6 +123,7 @@ SIGNATURES = {
   'il_fill_normal': (C.c_int, [vp, vp, i64, u64, u64, vp, vp]),
   'il_fill_uniform': (C.c_int, [vp, vp, i64, u64, u64, vp, vp]),
   'il_counter_add': (C.c_int, [vp, vp, u64, vp]),
+  'il_replica_copy': (C.c_int, [vp, C.c_int, P(vp), P(i64), P(i64), C.c_int, vp, vp]),
   'il_actor_workspace_bytes': (i64, [P(Mlp), C.c_int, C.c_int]),
   'il_actor_forward': (C.c_int, [vp, P(Mlp), C.c_int, C.c_int, vp, i64, C.c_int, vp, vp, vp, vp, vp, vp, vp, i64, vp]),
   'il_critic_workspace_bytes': (i64, [P(Mlp), C.c_int, C.c_int]),

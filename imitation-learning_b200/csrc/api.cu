@@ -9,7 +9,7 @@ int gemm_init();
 int mlp_init();
 
 extern "C" const char* il_last_error(void) { return g_il_error; }
-extern "C" int il_version(void) { return 101; }
+extern "C" int il_version(void) { return 102; }
 
 extern "C" int il_create(int device, il_handle** out) {
   IL_CHECK(out != nullptr, "il_create: null out");

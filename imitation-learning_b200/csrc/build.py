@@ -4,7 +4,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ['api.cu', 'gemm.cu', 'tc_gemm.cu', 'mlp.cu', 'sac.cu', 'replay.cu', 'env.cu', 'eval.cu', 'gail.cu', 'gail_general.cu', 'dropout_nets.cu', 'gmmil_pwil.cu']
+SOURCES = ['api.cu', 'gemm.cu', 'tc_gemm.cu', 'mlp.cu', 'sac.cu', 'replay.cu', 'env.cu', 'eval.cu', 'gail.cu', 'gail_general.cu', 'dropout_nets.cu', 'gmmil_pwil.cu', 'replica.cu']
 LIB = os.path.join(HERE, 'libil_b200.so')
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
 FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr']

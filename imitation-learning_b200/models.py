@@ -587,13 +587,20 @@ class PWILDiscriminator:
     self.data_scale, self.data_offset = (1 / inv_scale).contiguous(), offset.contiguous()
     self.atoms = (self.data_scale * (atoms + self.data_offset)).contiguous()  # :229
     self.reward_scale = imitation_cfg.reward_scale if reward_scale is None else reward_scale
-    scale = imitation_cfg.reward_bandwidth_scale if reward_bandwidth_scale is None else reward_bandwidth_scale
-    if per_replica(scale, 'cpu') is not None: scale = per_replica(scale, 'cpu', torch.float64)  # the host expression below in double, replica by replica
-    self.reward_bandwidth = scale * time_horizon / sqrt(state_size if self.state_only else state_size + action_size)  # :222
+    self.reward_bandwidth = self._bandwidth(imitation_cfg.reward_bandwidth_scale if reward_bandwidth_scale is None else reward_bandwidth_scale)
     self.reward_scale_r, self.reward_bandwidth_r = per_replica(self.reward_scale, self.device), per_replica(self.reward_bandwidth, self.device)
     for t in (self.reward_scale_r, self.reward_bandwidth_r): assert t is None or t.numel() == replicas, 'one PWIL reward scale / bandwidth per replica'
     self.expert_weights = torch.empty(replicas, self.atoms.size(0), device=self.device)
     self.reset()
+
+  def _bandwidth(self, scale):
+    if per_replica(scale, 'cpu') is not None: scale = per_replica(scale, 'cpu', torch.float64)  # the host expression below in double, replica by replica
+    return scale * self.time_horizon / sqrt(self.state_size if self.state_only else self.state_size + self.action_size)  # :222
+
+  def set_reward_hparams(self, reward_scale=None, reward_bandwidth_scale=None):
+    """Rewrites the per-replica reward scale / bandwidth arrays in place (same expressions as the constructor); None leaves one as it is."""
+    if reward_scale is not None: self.reward_scale_r.copy_(per_replica(reward_scale, self.device))
+    if reward_bandwidth_scale is not None: self.reward_bandwidth_r.copy_(per_replica(self._bandwidth(reward_bandwidth_scale), self.device))
 
   def _get_expert_atoms(self) -> Tensor:  # :225-226
     s, a = self.expert_memory['states'], self.expert_memory['actions']

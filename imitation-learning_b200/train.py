@@ -57,16 +57,18 @@ def check_config(cfg: Config):
 
 
 class Trainer:
-  def __init__(self, cfg: Config, replicas: Optional[int] = None, seed_offset: int = 0, fast_init: bool = False, device=None, hparams: Optional[Dict[str, Tensor]] = None):
+  def __init__(self, cfg: Config, replicas: Optional[int] = None, seed_offset: int = 0, fast_init: bool = False, device=None, hparams: Optional[Dict[str, Tensor]] = None,
+               grad_penalty_any: Optional[bool] = None):
     """hparams: {key: [R] values} of per-replica hyperparameters (the keys of sweep.BATCHABLE); replica r trains with its own values and
-    equals, bit for bit, a run configured with them. Without it every replica uses the config's values."""
+    equals, bit for bit, a run configured with them. Without it every replica uses the config's values. They can be changed in place later
+    (set_hparams). grad_penalty_any: whether any replica may ever have a positive imitation.grad_penalty (default: any initial value > 0);
+    it decides at set-up whether the penalty noise is drawn and whether the general discriminator runs its penalty pass."""
     check_config(cfg)
     self.cfg = cfg
     self.R = R = int(cfg.get('replicas', 1) if replicas is None else replicas)
     self.device = dev = torch.device('cuda', torch.cuda.current_device()) if device is None else torch.device(device)
     self.hparams = self._check_hparams(hparams or {}, cfg, R, dev)
     hp = lambda key, default: self.hparams.get(key, default)  # float64 [R] (the optimisers keep lr / weight decay in double) or the config float
-    hp32 = lambda key, default: self.hparams[key].float() if key in self.hparams else default  # float scalars of the kernels, rounded like a Python float
     self.lib, self.h = _lib.lib(), _lib.handle(dev.index)
     _lib.check(self.lib.il_set_gemm_mode(self.h, _lib.GEMM_MODE[cfg.get('gemm_mode', 'fp32')]))
     self.seed = seed = cfg.seed + seed_offset
@@ -82,20 +84,20 @@ class Trainer:
     need_expert = self.algorithm != 'SAC' or cfg.bc_pretraining.iterations > 0 or cfg.imitation.bc_aux_loss
     self.expert_memory = self.env.get_dataset(trajectories=cfg.imitation.trajectories, subsample=cfg.imitation.subsample) if need_expert else None
     self.S, self.A = S, A = self.env.observation_space.shape[0], self.env.action_space.shape[0]
+    derived = self._derived_hparams()
     # train.py:64-67 — replica r draws its initial weights from the stream of seed + r (fast_init: one stream, replicated)
     rng = None if (R == 1 or fast_init) else ReplicaRNG(seed, R)
     nrep = 1 if fast_init else R
     self.actor, self.critic = SoftActor(S, A, cfg.reinforcement.actor, replicas=nrep, rng=rng, device=dev), TwinCritic(S, A, cfg.reinforcement.critic, replicas=nrep, rng=rng, device=dev)
     self.discriminator = None
-    self.discount, self.polyak = hp32('reinforcement.discount', cfg.reinforcement.discount), hp32('reinforcement.polyak_factor', cfg.reinforcement.polyak_factor)
+    self.discount, self.polyak = derived['discount'], derived['polyak']
     if self.algorithm == 'GAIL': self.discriminator = GAILDiscriminator(S, A, cfg.imitation, self.discount, replicas=nrep, rng=rng, device=dev)
     elif self.algorithm == 'DRIL': self.discriminator = SoftActor(S, A, cfg.imitation.discriminator, replicas=nrep, rng=rng, device=dev)  # train.py:74
     elif self.algorithm == 'RED': self.discriminator = REDDiscriminator(S, A, cfg.imitation, replicas=nrep, rng=rng, device=dev)  # train.py:82
     if fast_init and R > 1: self._replicate()
     self.log_alpha = torch.zeros(R, device=dev)
     self.target_critic = create_target_network(self.critic)
-    tt = hp('reinforcement.target_temperature', cfg.reinforcement.target_temperature)
-    self.entropy_target = (tt * A).float() if isinstance(tt, Tensor) else tt * A
+    self.entropy_target = derived['entropy_target']
     lr, wd = hp('training.learning_rate', cfg.training.learning_rate), hp('training.weight_decay', cfg.training.weight_decay)
     self.actor_optimiser, self.critic_optimiser = AdamW(self.actor.parameters(), lr=lr, weight_decay=wd), AdamW(self.critic.parameters(), lr=lr, weight_decay=wd)
     self.temperature_optimiser = Adam([self.log_alpha], lr=lr)
@@ -142,8 +144,13 @@ class Trainer:
     self.sac_out = dict(log_probs=f(R, B), q_values=f(R, B), losses=f(R, 3))
     self.gail_losses = f(R, 2)
     self.rng = _RNG(seed, dev)
-    self.grad_penalty, self.entropy_bonus = hp32('imitation.grad_penalty', None), hp32('imitation.entropy_bonus', None)
-    self.grad_penalty_any = bool((self.hparams['imitation.grad_penalty'] > 0).any()) if 'imitation.grad_penalty' in self.hparams else None  # set-up time, never in a capture
+    self.grad_penalty, self.entropy_bonus = derived['grad_penalty'], derived['entropy_bonus']
+    self.grad_penalty_any = None
+    if 'imitation.grad_penalty' in self.hparams:  # set-up time, never in a capture
+      positive = bool((self.hparams['imitation.grad_penalty'] > 0).any())
+      if grad_penalty_any is False and positive: raise ValueError('grad_penalty_any=False but some replica starts with imitation.grad_penalty > 0')
+      self.grad_penalty_any = positive if grad_penalty_any is None else bool(grad_penalty_any)
+    self._src_of = None  # exploit(): the device replica map, allocated on first use and rewritten in place
     self.inject = False  # tests: True = all noise / index buffers are filled by the caller before each step
     self.dril_masks = None  # tests (inject): the dropout masks of this step's DRIL ensemble pass
     self.device_rng = bool(cfg.get('device_rng', True))
@@ -177,6 +184,84 @@ class Trainer:
       if k in ('imitation.grad_penalty', 'imitation.entropy_bonus') and not bool((host >= 0).all()): raise ValueError(f'hparams: {k} must be >= 0')
       out[k] = t.to(dev).contiguous()
     return out
+
+  def _derived_hparams(self) -> Dict[str, object]:
+    """The float32 kernel arguments computed from self.hparams (a [R] device array for a per-replica key, else the config's scalar or None):
+    the constructor creates them and set_hparams rewrites them in place, through this one function."""
+    cfg, hps = self.cfg, self.hparams
+    hp32 = lambda key, default: hps[key].float() if key in hps else default  # float scalars of the kernels, rounded like a Python float
+    tt = hps.get('reinforcement.target_temperature', cfg.reinforcement.target_temperature)
+    A = self.A
+    return dict(discount=hp32('reinforcement.discount', cfg.reinforcement.discount), polyak=hp32('reinforcement.polyak_factor', cfg.reinforcement.polyak_factor),
+                entropy_target=(tt * A).float() if isinstance(tt, Tensor) else tt * A,
+                grad_penalty=hp32('imitation.grad_penalty', None), entropy_bonus=hp32('imitation.entropy_bonus', None))
+
+  def set_hparams(self, values: Dict[str, object]):
+    """Writes new [R] values of per-replica hyperparameters in place: self.hparams, every float32 array derived from them and the arrays the
+    optimisers hold. Nothing is allocated that a kernel reads, so captured CUDA graphs keep running, now with the new values. Only keys the
+    trainer was built with can change (a key set up as a scalar is baked into the graphs)."""
+    new = self._check_hparams(values, self.cfg, self.R, self.device)
+    fixed = [k for k in new if k not in self.hparams]
+    if fixed: raise ValueError(f'set_hparams: {", ".join(fixed)} was not per-replica at construction (Trainer(hparams=...)); per-replica keys: {", ".join(self.hparams) or "none"}')
+    if 'imitation.grad_penalty' in new and not self.grad_penalty_any and bool((new['imitation.grad_penalty'] > 0).any()):
+      raise ValueError('set_hparams: a positive imitation.grad_penalty needs Trainer(grad_penalty_any=True): this trainer was set up without the penalty draws')
+    for k, v in new.items(): self.hparams[k].copy_(v)
+    for name, v in self._derived_hparams().items():
+      cur = getattr(self, name)
+      if isinstance(cur, Tensor): cur.copy_(v)
+    if self.algorithm == 'PWIL': self.discriminator.set_reward_hparams(self.hparams.get('imitation.reward_scale'), self.hparams.get('imitation.reward_bandwidth_scale'))
+    for name, (lr_key, wd_key) in (('actor_optimiser', ('training.learning_rate', 'training.weight_decay')), ('critic_optimiser', ('training.learning_rate', 'training.weight_decay')),
+                                   ('temperature_optimiser', ('training.learning_rate', None)),
+                                   ('discriminator_optimiser', ('imitation.learning_rate', 'imitation.weight_decay'))):
+      opt = getattr(self, name, None)
+      if opt is None: continue
+      for arr, key in ((opt.lr_r, lr_key), (opt.weight_decay_r, wd_key)):
+        if arr is not None and key in self.hparams and arr.data_ptr() != self.hparams[key].data_ptr(): arr.copy_(self.hparams[key])
+
+  def replica_state(self) -> List[Tensor]:
+    """Every tensor whose leading axis is the replica axis and that carries training state from one step to the next: network, target and
+    optimiser state, log_alpha, the discriminator's learned and set-up state, the replay ring and its counters, the environments and the loop's
+    episode bookkeeping. Excluded: values shared by all replicas (step counts, RNG counters, AdRIL's flag, the expert memory), workspaces,
+    noise and index buffers and per-call outputs, which are rewritten before they are read."""
+    out = [self.actor.mlp.flat, self.critic.mlp.flat, self.target_critic.mlp.flat, self.log_alpha]
+    for name in ('actor_optimiser', 'critic_optimiser', 'temperature_optimiser', 'discriminator_optimiser'):
+      opt = getattr(self, name, None)
+      if opt is not None: out += [opt.exp_avg, opt.exp_avg_sq]
+    d = self.discriminator
+    if self.algorithm == 'GAIL':
+      out += [d.flat, d.g_u, d.g_v, d.h_u, d.h_v] if d.general else [d.mlp.flat, d.u, d.v]
+    elif self.algorithm == 'DRIL': out += [d.mlp.flat, d._q if d.q is not None else None]
+    elif self.algorithm == 'RED': out += [d.predictor.flat, d.target.flat, d.sigma]
+    elif self.algorithm == 'PWIL': out += [d.expert_weights]
+    elif self.algorithm == 'GMMIL': out += [d.gamma]
+    m = self.memory
+    out += [m.rows, m._idx, m._full, m._num_trajectories, self.env.batch.x, self.env.batch.t]
+    out += [self.state, self.step_f, self.running_return, self.last_return, self.return_sum, self.episodes]
+    return [t for t in out if t is not None]
+
+  def exploit(self, src_of):
+    """Population-based training's exploit step: replica r becomes a copy of replica src_of[r] (a host [R] map, or {destination: source}) in
+    every tensor of replica_state() and every per-replica hyperparameter, with one il_replica_copy launch. A source must be its own source.
+    A destination keeps its seed and its position in the noise buffers, so afterwards it differs from its source only in the noise it draws."""
+    R = self.R
+    if isinstance(src_of, dict):
+      m = np.arange(R)
+      for dst, src in src_of.items(): m[int(dst)] = int(src)
+    else: m = np.asarray(src_of).reshape(-1)
+    if m.shape != (R, ) or not np.issubdtype(m.dtype, np.integer) or m.min() < 0 or m.max() >= R:
+      raise ValueError(f'exploit: expected {R} replica indices in [0, {R}), got {src_of!r}')
+    m = m.astype(np.int32)
+    if not np.array_equal(m[m], m): raise ValueError(f'exploit: replicas {np.flatnonzero(m[m] != m).tolist()} copy from a replica that is itself overwritten')
+    if self._src_of is None: self._src_of = torch.empty(R, dtype=torch.int32, device=self.device)
+    self._src_of.copy_(torch.from_numpy(m))
+    bufs = self.replica_state()
+    for t in bufs: assert t.size(0) == R and t.is_contiguous() and t.element_size() == 4, 'replica_state(): contiguous 4-byte [R, ...] buffers'
+    n = len(bufs)
+    base = (C.c_void_p * n)(*[t.data_ptr() for t in bufs])
+    stride = (C.c_int64 * n)(*[t.stride(0) * 4 for t in bufs])
+    nbytes = (C.c_int64 * n)(*[t[0].numel() * 4 for t in bufs])
+    _lib.check(self.lib.il_replica_copy(self.h, n, base, stride, nbytes, R, self._src_of.data_ptr(), _lib.stream()))
+    if self.hparams: self.set_hparams({k: v.cpu()[torch.from_numpy(m).long()] for k, v in self.hparams.items()})
 
   def _pwil_relabel_expert(self):
     """train.py:136-140: the expert's own transitions get their greedy PWIL reward, walking the expert memory in order and
@@ -414,18 +499,29 @@ def train(cfg: Config, file_prefix: str = '') -> float:
   total = int(cfg.get('replicas', 1))
   lo, hi = distributed.shard(total, rank, world)
   keys, values = sweep.setup(cfg)  # hyperparameter search on the replica axis (sweep.space / sweep.trials)
-  hparams, sweep_sums = None, []
+  pbt = sweep.pbt_config(cfg, world)  # population-based training on top of it (sweep.pbt.*); None when off
+  hparams, sweep_sums, pbt_records, initial_values = None, [], [], values
   if values is not None:
     hparams = sweep.shard(sweep.replica_hparams(keys, values, total), lo, hi)
     trials_here = sweep.trial_of(total, len(values))[lo:hi]
-  trainer = Trainer(cfg, replicas=hi - lo, seed_offset=lo, hparams=hparams)
+  trainer = Trainer(cfg, replicas=hi - lo, seed_offset=lo, hparams=hparams, grad_penalty_any=None if pbt is None else pbt['grad_penalty_any'])
   metrics, score = trainer.metrics, trainer.score
 
-  def sweep_eval(normalized):
-    if values is not None: sweep_sums.append(sweep.reduce_sums(sweep.trial_sums(normalized, trials_here, len(values))))
+  def sweep_eval(normalized, step):
+    nonlocal values
+    if values is None: return
+    sweep_sums.append(sweep.reduce_sums(sweep.trial_sums(normalized, trials_here, len(values))))
+    if pbt is not None and len(sweep_sums) % pbt['interval'] == 0 and step + cfg.evaluation.interval <= cfg.steps:  # the final evaluation ranks, it does not exploit
+      scores_now = sweep.latest_scores(sweep_sums, len(values))
+      parents, values = sweep.pbt_step(pbt, keys, values, scores_now, len(pbt_records))
+      trainer.exploit(sweep.replica_map(parents, total)[lo:hi] - lo)  # rank-local: every source of this rank's replicas lives on this rank
+      trainer.set_hparams(sweep.shard(sweep.replica_hparams(keys, values, total), lo, hi))
+      pbt_records.append(dict(step=step, parents=parents, values=values, scores=scores_now))
 
   def sweep_save():
-    if values is not None and rank == 0: sweep.write_results(file_prefix, keys, values, total // len(values), sweep.scores(sweep_sums, len(values)))
+    if values is None or rank != 0: return
+    if pbt is None: sweep.write_results(file_prefix, keys, values, total // len(values), sweep.scores(sweep_sums, len(values)))
+    else: sweep.write_results(file_prefix, keys, values, total // len(values), sweep.latest_scores(sweep_sums, len(values)), pbt=dict(initial=initial_values, records=pbt_records))
   start_time = time.time()
   if cfg.bc_pretraining.iterations > 0:  # train.py:93-112
     trainer.bc_pretrain()
@@ -433,7 +529,7 @@ def train(cfg: Config, file_prefix: str = '') -> float:
       returns = trainer.evaluate()
       mean, std, n = distributed.return_statistics(returns)
       normalized = (returns.cpu().numpy() - trainer.normalization_min) / (trainer.normalization_max - trainer.normalization_min)
-      sweep_eval(normalized)
+      sweep_eval(normalized, 0)
       sweep_save()
       flat = total == 1
       metrics['test_steps'], metrics['test_returns'], metrics['test_returns_normalized'] = [0], [returns.cpu().numpy().reshape(-1).tolist() if flat else returns.cpu().numpy().tolist()], \
@@ -452,7 +548,7 @@ def train(cfg: Config, file_prefix: str = '') -> float:
       mean, std, n = distributed.return_statistics(returns)
       normalized = (returns.cpu().numpy() - trainer.normalization_min) / (trainer.normalization_max - trainer.normalization_min)
       score.append(float((mean - trainer.normalization_min) / (trainer.normalization_max - trainer.normalization_min)))
-      sweep_eval(normalized)
+      sweep_eval(normalized, step)
       metrics['test_steps'].append(step)
       flat = total == 1  # the reference's schema: one list of `episodes` floats per evaluation (train.py:214-219); R > 1 keeps [R][episodes]
       metrics['test_returns'].append(returns.cpu().numpy().reshape(-1).tolist() if flat else returns.cpu().numpy().tolist())

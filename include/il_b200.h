@@ -118,6 +118,17 @@ int il_fill_normal(il_handle* h, float* out, int64_t n, uint64_t seed, uint64_t 
 int il_fill_uniform(il_handle* h, float* out, int64_t n, uint64_t seed, uint64_t stream_id, const uint64_t* counter, void* stream);
 int il_counter_add(il_handle* h, uint64_t* counter, uint64_t inc, void* stream);
 
+/* ---- replica state copy (population-based training, sweep.py) ------------------------------------------ */
+/* For every buffer b and every replica r with src_of[r] != r: copy bytes[b] bytes from base[b] + src_of[r] * stride_bytes[b] to
+ * base[b] + r * stride_bytes[b]. src_of is a device [R] int32 map; it may change between replays of a captured call (identity entries
+ * cost one read of the map). Host arrays of nbufs <= IL_REPLICA_COPY_MAX_BUFS entries; every base, stride and length 4-byte aligned,
+ * bytes <= stride (16-byte aligned buffers take the vector path).
+ * Precondition (the caller guarantees it; documented, not checked on the device): every source is its own source, i.e.
+ * src_of[src_of[r]] == src_of[r], so no replica is both read and written. */
+#define IL_REPLICA_COPY_MAX_BUFS 64
+int il_replica_copy(il_handle* h, int nbufs, void* const* base, const int64_t* stride_bytes, const int64_t* bytes, int R, const int32_t* src_of,
+                    void* stream);
+
 /* ---- SoftActor (models.py:84-102) --------------------------------------------------------------------- */
 /* forward + tanh-Gaussian head for n states per replica. eps == NULL: greedy (tanh(mean), models.py:101-102).
  * eps != NULL: action = tanh(mean + std*eps) and log_prob via the cached pre-tanh value (train.py:152,
